@@ -2,7 +2,7 @@
 """bench.py -- queries/sec of the DeltaPQ query hot path (ADC tables -> DeltaTree scan ->
 top-k) on B200, through libdpq.so's C ABI (include/dpq.h).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): SIFT1M-shaped synthetic, 1M x 128-d, M=8 K=256 h=1,
 10K queries, top-10.  One step = one pass of the hot path over one batch of 10K queries.
@@ -211,6 +211,25 @@ def timed_steps(torch, stream, flush, steps, step_fn, barrier):
     return float(sum(a.elapsed_time(b) for a, b in ev))
 
 
+def dump_outputs(out_dir, pos, ids, dist):
+    """--dump-outputs: the top-k of the last timed step (all queries, rank 0's batch), as a caller of
+    dpq_index_search receives it: DFS positions, vector ids (float64: every uint32 is exact) and
+    distances (float32, as computed), one row per query in ascending distance.  Past 64 MB in all, a
+    fixed seeded sample of the queries is kept and query_rows.npy names them.  The inputs are seeded,
+    so two builds run with the same arguments can be compared array by array."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"positions": np.asarray(pos, np.float64), "ids": np.asarray(ids, np.float64),
+              "distances": np.asarray(dist, np.float32)}
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    max_rows = (64_000_000 - 4096) // (row_bytes + 8)  # 4 KB for the .npy headers
+    if len(pos) > max_rows:
+        rows = np.sort(np.random.default_rng(0).choice(len(pos), max_rows, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["query_rows"] = rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_gpu(args):
     import torch
     import deltapq_b200 as dpq
@@ -329,6 +348,8 @@ def run_gpu(args):
     out_pos, out_dist = dpq.unpack_keys(d_key.cpu().numpy().view(np.uint64))
     assert np.all(np.diff(out_dist.astype(np.float64), axis=1) >= 0), "top-k not ascending"
     assert np.array_equal(out_dist, dst) and np.array_equal(out_pos, pos), "device and host paths disagree"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_pos, ids, out_dist)
 
     # ---- secondary mode at N > 1: the SAME tree sharded by depth-1 subtrees over the ranks
     # (SURVEY 8e, the 1B-code design): every rank scans its shard for the same 10K queries, one
@@ -381,7 +402,7 @@ def run_gpu(args):
                 qn.tofile(os.path.join(tmpd, "qnodes.bin"))
                 del qn
                 np.savez(os.path.join(tmpd, "multi_probe.npz"), cw=cw, queries=queries0, topk=k, n_codes=args.n_codes)
-                r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "multi_probe.py"), tmpd, str(world), "5"],
+                r = subprocess.run([sys.executable, "-B", os.path.join(ROOT, "tools", "multi_probe.py"), tmpd, str(world), "5"],
                                    capture_output=True, text=True, timeout=420)
                 last = [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
                 multi_cpp = json.loads(last[-1]) if last else {"error": (r.stderr or r.stdout)[-300:], "rc": r.returncode}
@@ -779,6 +800,7 @@ class StdoutToStderr:
 
 
 def main():
+    sys.dont_write_bytecode = True  # the bench leaves the source tree as it found it (it may be read-only)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -796,7 +818,13 @@ def main():
     ap.add_argument("--c5-steps", type=int, default=3)
     ap.add_argument("--c5-check-queries", type=int, default=4)
     ap.add_argument("--c5-ref-queries", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the top-k of the last timed step to DIR/{positions,ids,distances}.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     if args.warmup < 3:
         args.warmup = 3
     holder = []

@@ -1,5 +1,6 @@
 import os, sys, time
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tests')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import numpy as np, datagen as dg, deltapq_b200 as dpq
 os.environ["DPQ_EDGE_STATS"] = "1"
 M = int(sys.argv[1]); N = int(sys.argv[2])
