@@ -106,6 +106,7 @@ struct dpq_index {
                                // full pass (0: none; -1 auto: 4 for the wide shape with topk > 32)
     int opt_presample = 0;     // nodes scored exactly per query to seed the sample pass (0 auto: 2048, or 4096 for topk > 32)
     int opt_bcap8 = 0, opt_warps8 = 24, opt_levels8 = 80;  // bcap8 0 = auto (512 narrow, 2048 wide)
+    int opt_reuse8 = 1;        // 1: the narrow coarse scan reads only the table rows whose code byte changed (scan8.cu); 0: all
     int opt_stight = 100;      // percent of the presample cap the first sampled pass accepts (100 = all of it)
     int64_t opt_coarse_min = 100000;  // nodes in the shard from which the coarse search pays (gpurun_out/probe22.log)
     int opt_dbg_bound = 0x8000;  // developer probe: initial exclusive bound (results are wrong below 0x8000)
@@ -586,6 +587,7 @@ int dpq_index_set_option(dpq_index* ix, const char* name, int64_t v) {
     else if (n == "sample") ix->opt_sample = std::max(0, (int)v);
     else if (n == "bcap8") ix->opt_bcap8 = v <= 0 ? 0 : std::max(32, (int)v);
     else if (n == "warps8") ix->opt_warps8 = std::max(2, std::min(24, (int)v));
+    else if (n == "reuse8") ix->opt_reuse8 = v != 0;
     else if (n == "coarse_min") ix->opt_coarse_min = v;
     else if (n == "seed") ix->opt_seed = (int)v;
     else if (n == "refine") ix->opt_refine = (int)v;
@@ -1021,6 +1023,7 @@ int dpq_index_search_device(dpq_index* ix, const float* d_queries, int Q, int to
         s8.bcap = bcap8;
         s8.thresh = levels8 + c8.slack + 1;
         s8.nf = c8.nf;
+        s8.reuse = ix->opt_reuse8;
         dpq::Rescore8Args r8;
         r8.cand = s8.cand;
         r8.cand_cnt = s8.cand_cnt;

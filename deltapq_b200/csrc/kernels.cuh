@@ -83,6 +83,16 @@ __device__ __forceinline__ uint2 lds64(uint32_t saddr) {
     asm volatile("ld.shared.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(saddr));
     return v;
 }
+// Loads only when `load` != 0; otherwise v keeps what it held (a skipped load sends no wavefront).
+// The test is written into the asm so that ptxas makes it one LOP3 with a predicate output.
+__device__ __forceinline__ void lds128_if(uint4& v, uint32_t saddr, uint32_t load) {
+    asm volatile(
+        "{\n.reg .pred p;\n"
+        "setp.ne.b32 p, %5, 0;\n"
+        "@p ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];\n}\n"
+        : "+r"(v.x), "+r"(v.y), "+r"(v.z), "+r"(v.w)
+        : "r"(saddr), "r"(load));
+}
 // hints: pull the line three lines ahead of the record cursor into L2 (hides HBM latency when the
 // tree does not fit L2; a 16M-code tree ran 3.4x off the shared-memory bound without it), and the
 // next line into L1
@@ -187,6 +197,7 @@ struct Scan8Args {
     int Q, n_groups, n_slices, n_warps, bcap;
     int thresh;                   // hit iff coarse sum < thresh (= levels + slack + 1 <= 128)
     int nf;                       // 8: narrow shape, 16: wide shape (C8Shape)
+    int reuse;                    // narrow shape, 1: a strand keeps its table rows and reads only those of changed code bytes
 };
 // coarse tables: entry = min(SAT, rint(lut / unit)), unit = cap / levels, cap = the query's exact k-th
 // distance over the sample; transposed to [group][m * 256 + centroid][112 queries]

@@ -199,7 +199,7 @@ void launch_pack8(const float* d_lutf, const float* d_cap, int M, int K, int Q, 
 //   NF = 8 : LDS.128 of the 112-byte row, word k byte b = query jj*16 + 4k + b
 //   NF = 16: LDS.64 of the 56-byte row (nibbles); sums E0, O0, E1, O1 = even / odd nibbles of the two
 //            loaded words: word w (k = w >> 1, parity p = w & 1) byte b = query jj*16 + 8k + 2b + p
-template <int NF>
+template <int NF, bool REUSE>
 __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
     constexpr int QB = 112;                      // queries per CTA
     constexpr int ROWS = NF * 256;
@@ -258,6 +258,18 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
     const CodeT* codes = reinterpret_cast<const CodeT*>(a.codes);
     constexpr int PF = 128 / (int)sizeof(CodeT);  // nodes per 128-byte line
 
+    // Row reuse (REUSE, narrow shape): a strand walks consecutive DFS positions, and a node often shares
+    // a centroid with the node before it in some subspaces (21 % of the rows of the 1M SIFT-shaped tree,
+    // tools/row_reuse_stats.py).  The eight rows stay in registers across nodes and a row is read only
+    // when its code byte changed: one LOP3 with a predicate output per row, and a skipped read sends no
+    // shared-memory wavefront for that strand.  The rows, and so the sums, are the same as when every
+    // row is read.  REUSE = false reads all of them every node.  The wide scan does not reuse rows: it
+    // is issue-bound, and the sixteen predicates made it slower (profiles/r3_summary.md).
+    static_assert(NF == 8 || !REUSE, "row reuse is narrow-shape only");
+    uint4 A[8];
+#pragma unroll
+    for (int r = 0; r < 8; ++r) A[r] = make_uint4(0u, 0u, 0u, 0u);
+
     for (int round = 0; round < n_rounds; ++round) {
         const int bt = b_lo + round * a.n_warps + warp;
         const int c = bt * a.bt_stride * SPW + strand;
@@ -270,6 +282,9 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
         }
         CodeT rec = CodeWord<NF>::zero(), nxt;
         if (n_nodes > 0) rec = __ldg(codes + nix);
+        // code bytes that differ from the strand's previous node: at a chunk start all of them, on an
+        // idle strand none (past a chunk's last node the code is 0: one read of the changed rows, then none)
+        uint2 chg = n_nodes > 0 ? make_uint2(~0u, ~0u) : make_uint2(0u, 0u);
 #pragma unroll 1
         for (int it = 0; it < C; ++it) {
             ++nix;
@@ -280,18 +295,15 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
             if (it + 1 < n_nodes) nxt = __ldg(codes + nix);
             uint32_t d[4];
             if constexpr (NF == 8) {
-                const uint4 A0 = lds128o<0 * SUB>(rowaddr<ROWB>(lut_base, rec.x, 0));
-                const uint4 A1 = lds128o<1 * SUB>(rowaddr<ROWB>(lut_base, rec.x, 1));
-                const uint4 A2 = lds128o<2 * SUB>(rowaddr<ROWB>(lut_base, rec.x, 2));
-                const uint4 A3 = lds128o<3 * SUB>(rowaddr<ROWB>(lut_base, rec.x, 3));
-                const uint4 A4 = lds128o<4 * SUB>(rowaddr<ROWB>(lut_base, rec.y, 0));
-                const uint4 A5 = lds128o<5 * SUB>(rowaddr<ROWB>(lut_base, rec.y, 1));
-                const uint4 A6 = lds128o<6 * SUB>(rowaddr<ROWB>(lut_base, rec.y, 2));
-                const uint4 A7 = lds128o<7 * SUB>(rowaddr<ROWB>(lut_base, rec.y, 3));
-                d[0] = (A0.x + A1.x + A2.x) + (A3.x + A4.x + A5.x) + (A6.x + A7.x);
-                d[1] = (A0.y + A1.y + A2.y) + (A3.y + A4.y + A5.y) + (A6.y + A7.y);
-                d[2] = (A0.z + A1.z + A2.z) + (A3.z + A4.z + A5.z) + (A6.z + A7.z);
-                d[3] = (A0.w + A1.w + A2.w) + (A3.w + A4.w + A5.w) + (A6.w + A7.w);
+                const uint32_t w2[2] = {rec.x, rec.y};
+                const uint32_t ch2[2] = {REUSE ? chg.x : ~0u, REUSE ? chg.y : ~0u};
+#pragma unroll
+                for (int r = 0; r < 8; ++r)
+                    lds128_if(A[r], rowaddr<ROWB>(lut_base, w2[r >> 2], r & 3) + (uint32_t)(r * SUB), ch2[r >> 2] & (0xFFu << (8 * (r & 3))));
+                d[0] = (A[0].x + A[1].x + A[2].x) + (A[3].x + A[4].x + A[5].x) + (A[6].x + A[7].x);
+                d[1] = (A[0].y + A[1].y + A[2].y) + (A[3].y + A[4].y + A[5].y) + (A[6].y + A[7].y);
+                d[2] = (A[0].z + A[1].z + A[2].z) + (A[3].z + A[4].z + A[5].z) + (A[6].z + A[7].z);
+                d[3] = (A[0].w + A[1].w + A[2].w) + (A[3].w + A[4].w + A[5].w) + (A[6].w + A[7].w);
             } else {
                 const uint32_t w4[4] = {rec.x, rec.y, rec.z, rec.w};
                 d[0] = d[1] = d[2] = d[3] = 0u;
@@ -331,6 +343,7 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
                     }
                 }
             }
+            if constexpr (REUSE) chg = make_uint2(nxt.x ^ rec.x, nxt.y ^ rec.y);
             rec = nxt;
             ++pos;
         }
@@ -343,7 +356,7 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
 cudaError_t launch_scan8(const Scan8Args& a, cudaStream_t st) {
     const C8Shape sh = c8_shape(a.nf);
     const size_t smem = (size_t)sh.lut_bytes() + 128 * 4 + 16;
-    void (*k)(const Scan8Args) = a.nf == 8 ? scan8_kernel<8> : scan8_kernel<16>;
+    void (*k)(const Scan8Args) = a.nf == 16 ? scan8_kernel<16, false> : a.reuse ? scan8_kernel<8, true> : scan8_kernel<8, false>;
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     k<<<(unsigned)(a.n_groups * a.n_slices), (unsigned)(a.n_warps * 32), smem, st>>>(a);
