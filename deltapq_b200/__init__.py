@@ -26,7 +26,7 @@ SYMBOLS = [
     "dpq_groundtruth_finish", "dpq_groundtruth_stat", "dpq_program_compile", "dpq_program_size", "dpq_program_copy",
     "dpq_program_free", "dpq_tree_build", "dpq_tree_from_edges", "dpq_tree_size", "dpq_tree_copy",
     "dpq_tree_free", "dpq_multi_open_file", "dpq_multi_set_codebook", "dpq_multi_search", "dpq_multi_stat",
-    "dpq_multi_close",
+    "dpq_multi_close", "dpq_index_delete", "dpq_index_undelete", "dpq_multi_delete", "dpq_multi_undelete",
 ]
 
 
@@ -108,6 +108,8 @@ def lib():
     L.dpq_multi_stat.argtypes = [vp, i32, C.c_char_p]
     L.dpq_multi_close.argtypes = [vp]
     L.dpq_multi_close.restype = None
+    for name in ("dpq_index_delete", "dpq_index_undelete", "dpq_multi_delete", "dpq_multi_undelete"):
+        getattr(L, name).argtypes = [vp, vp, i64]
     _lib = L
     return L
 
@@ -169,6 +171,11 @@ def pinned_array(shape, dtype):
 
 
 _PINNED = []
+
+
+def _id_array(ids):
+    ids = np.ascontiguousarray(np.asarray(ids).reshape(-1), np.uint32)
+    return ids, (_ptr(ids) if ids.size else None)
 
 
 def unpack_keys(keys):
@@ -239,6 +246,15 @@ class DeltaTreeIndex:
         _check(lib().dpq_index_search(self._h, _ptr(q), Q, topk, _ptr(pos), _ptr(ids), _ptr(dist)))
         return pos, ids, dist
 
+    def delete(self, ids):
+        """dpq_index_delete: the vector ids (what search reports as ids) stop appearing in results."""
+        ids, p = _id_array(ids)
+        _check(lib().dpq_index_delete(self._h, p, ids.size))
+
+    def undelete(self, ids):
+        ids, p = _id_array(ids)
+        _check(lib().dpq_index_undelete(self._h, p, ids.size))
+
     def search_device(self, d_queries_ptr, Q, topk, d_out_ptr):
         _check(lib().dpq_index_search_device(self._h, d_queries_ptr, Q, topk, d_out_ptr))
 
@@ -283,6 +299,15 @@ class MultiIndex:
         dist = np.empty((Q, topk), np.float32)
         _check(lib().dpq_multi_search(self._h, _ptr(q), Q, topk, _ptr(pos), _ptr(ids), _ptr(dist)))
         return pos, ids, dist
+
+    def delete(self, ids):
+        """dpq_multi_delete: vector ids (through the QNode file when one was given, else positions)."""
+        ids, p = _id_array(ids)
+        _check(lib().dpq_multi_delete(self._h, p, ids.size))
+
+    def undelete(self, ids):
+        ids, p = _id_array(ids)
+        _check(lib().dpq_multi_undelete(self._h, p, ids.size))
 
     def stat(self, rank, name):
         return int(lib().dpq_multi_stat(self._h, rank, name.encode()))

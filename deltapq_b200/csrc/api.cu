@@ -120,6 +120,11 @@ struct dpq_index {
     int last_launches = 0;
     int64_t last_fallback = 0;
     bool timing_valid = false;
+    // deleted nodes: one bit per local position (null until the first dpq_index_delete = nothing deleted)
+    DevBuf d_dead, d_del_ids, d_del_tmp;
+    int64_t n_deleted = 0;
+    int64_t last_delete_us = 0;  // host wall clock of the last dpq_index_delete / _undelete (ends in a stream sync)
+    const uint32_t* dead() const { return d_dead.p ? d_dead.as<uint32_t>() : nullptr; }
 };
 
 namespace {
@@ -601,6 +606,62 @@ int dpq_index_set_option(dpq_index* ix, const char* name, int64_t v) {
     return DPQ_OK;
 }
 
+// dpq_index_delete / dpq_index_undelete: the ids are sorted on the device, then every 32-position word of the
+// bitmap is rebuilt from a binary search of its nodes' ids (dead.cu).  The caller's stream orders the change
+// before every later search; the call returns once it is complete.
+static int mark_dead(dpq_index* ix, const uint32_t* ids, int64_t n, bool set, const char* what) {
+    const auto t0 = std::chrono::steady_clock::now();
+    int rc = check_device();
+    if (rc) return rc;
+    if (!ix) return fail(DPQ_ERR_ARG, std::string(what) + ": null index");
+    if (n < 0 || (n > 0 && !ids)) return fail(DPQ_ERR_ARG, std::string(what) + ": ids is null or n < 0");
+    if (n > 0x7FFFFFFFLL) return fail(DPQ_ERR_ARG, std::string(what) + ": more than 2^31 - 1 ids in one call");
+    const dpq::ScanProgram& P = ix->prog;
+    if (!P.v2)
+        return fail(DPQ_ERR_ARG, std::string(what) +
+                                     ": deletion needs the code-array engine (this index runs the first-generation engine, DPQ_ENGINE=1)");
+    if (n == 0 || (!set && !ix->d_dead.p)) {
+        ix->last_delete_us = 0;
+        return DPQ_OK;
+    }
+    CU(cudaSetDevice(ix->device));
+    cudaStream_t st = ix->stream;
+    const size_t words = (size_t)((P.n_local + 31) / 32);
+    if (!ix->d_dead.p) {  // first delete: the bitmap appears, all live
+        if ((rc = ix->d_dead.ensure(std::max<size_t>(words, 1) * 4))) return rc;
+        CU(cudaMemsetAsync(ix->d_dead.p, 0, ix->d_dead.cap, st));
+    }
+    if (ix->has_pos2id && !ix->d_pos2id.p) {  // the same id table the host-buffer search uploads
+        if ((rc = ix->d_pos2id.ensure(std::max<size_t>(ix->pos2id_host.size(), 1) * 4))) return rc;
+        CU(cudaMemcpyAsync(ix->d_pos2id.p, ix->pos2id_host.data(), ix->pos2id_host.size() * 4, cudaMemcpyHostToDevice, st));
+    }
+    // [n raw ids][n sorted ids][count], then the sort's scratch
+    const size_t ids_bytes = ((size_t)n * 4 + 15) / 16 * 16;
+    size_t tmp_bytes = 0;
+    CU(dpq::sort_ids(nullptr, nullptr, (int)n, nullptr, &tmp_bytes, st));
+    if ((rc = ix->d_del_ids.ensure(2 * ids_bytes + 16)) || (rc = ix->d_del_tmp.ensure(std::max<size_t>(tmp_bytes, 16)))) return rc;
+    uint32_t* d_raw = ix->d_del_ids.as<uint32_t>();
+    uint32_t* d_sorted = reinterpret_cast<uint32_t*>(ix->d_del_ids.as<char>() + ids_bytes);
+    unsigned long long* d_count = reinterpret_cast<unsigned long long*>(ix->d_del_ids.as<char>() + 2 * ids_bytes);
+    CU(cudaMemcpyAsync(d_raw, ids, (size_t)n * 4, cudaMemcpyHostToDevice, st));
+    CU(dpq::sort_ids(d_raw, d_sorted, (int)n, ix->d_del_tmp.p, &tmp_bytes, st));
+    CU(cudaMemsetAsync(d_count, 0, 8, st));
+    dpq::launch_mark_dead(d_sorted, n, ix->has_pos2id ? ix->d_pos2id.as<uint32_t>() : nullptr, (uint32_t)P.base_pos, P.n_local, set,
+                          ix->d_dead.as<uint32_t>(), d_count, st);
+    CU(cudaGetLastError());
+    unsigned long long count = 0;
+    CU(cudaMemcpyAsync(&count, d_count, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    ix->n_deleted = (int64_t)count;
+    if (count == 0) ix->d_dead.release();  // nothing deleted: the searches are back on the kernels without liveness tests
+    ix->last_delete_us =
+        (int64_t)std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t0).count();
+    return DPQ_OK;
+}
+
+int dpq_index_delete(dpq_index* ix, const uint32_t* ids, int64_t n) { return mark_dead(ix, ids, n, true, "dpq_index_delete"); }
+int dpq_index_undelete(dpq_index* ix, const uint32_t* ids, int64_t n) { return mark_dead(ix, ids, n, false, "dpq_index_undelete"); }
+
 // slices of a pass over n_chunks chunks for n_groups query groups: whole waves of 148 one-CTA SMs and
 // whole rounds (warps x strands chunks) per item, as nearly as possible
 static int pick_slices(int n_groups, int n_chunks, int chunks_per_round, int max_slices) {
@@ -668,7 +729,8 @@ static int search_latency(dpq_index* ix, const float* d_queries, int Q, int topk
     float* cap0 = ix->d_cap0.as<float>();
     float* cap1 = ix->d_cap1.as<float>();
     if ((rc = ensure_sample_codes(ix, 2048))) return rc;
-    dpq::launch_presample(ix->d_lutf.as<float>(), ix->d_ps_codes.as<uint8_t>(), P.cstride, P.n_local, P.M, P.K, Q, topk, 2048, cap0, st);
+    dpq::launch_presample(ix->d_lutf.as<float>(), ix->d_ps_codes.as<uint8_t>(), P.cstride, P.n_local, P.M, P.K, Q, topk, 2048, cap0,
+                          ix->dead(), st);
     launches += 2;
     uint32_t* cnt = ix->d_cnt1.as<uint32_t>();  // [0..Q) counts, [Q..2Q) overflow flags; a second pair behind for the final pass
     dpq::Scan1Args s1;
@@ -683,6 +745,7 @@ static int search_latency(dpq_index* ix, const float* d_queries, int Q, int topk
     s1.n_pairs = (Q + 1) / 2;
     s1.cand = ix->d_cand1.as<uint32_t>();
     s1.ccap = ccap;
+    s1.dead = ix->dead();
     dpq::Rescore1Args r1;
     r1.cand = s1.cand;
     r1.ccap = ccap;
@@ -764,6 +827,7 @@ static int search_latency(dpq_index* ix, const float* d_queries, int Q, int topk
     fb.topk = topk;
     fb.part = ix->d_fpart.as<uint64_t>();
     fb.out_key = d_out_key;
+    fb.dead = ix->dead();
     dpq::launch_fallback(fb, st);
     launches += 4;
     CU(cudaEventRecord(ix->ev[3], st));
@@ -951,6 +1015,7 @@ int dpq_index_search_device(dpq_index* ix, const float* d_queries, int Q, int to
         s2.trigger = ix->opt_trigger > 0 ? std::min(ix->opt_trigger, g.bcap / 2) : std::min(2 * g.kp, g.bcap / 2);
         s2.epoch = std::max(1, ix->opt_epoch);
         s2.ramp = ix->opt_ramp;
+        s2.dead = ix->dead();
         CU(dpq::launch_scan2(s2, st));
         ++launches;
     } else if (!seeded) {
@@ -1003,6 +1068,7 @@ int dpq_index_search_device(dpq_index* ix, const float* d_queries, int Q, int to
     fa.topk = topk;
     fa.part = ix->d_fpart.as<uint64_t>();
     fa.out_key = d_out_key;
+    fa.dead = ix->dead();
     if (!coarse) {
         dpq::launch_fallback(fa, st);
         launches += 2;
@@ -1024,6 +1090,7 @@ int dpq_index_search_device(dpq_index* ix, const float* d_queries, int Q, int to
         s8.thresh = levels8 + c8.slack + 1;
         s8.nf = c8.nf;
         s8.reuse = ix->opt_reuse8;
+        s8.dead = ix->dead();
         dpq::Rescore8Args r8;
         r8.cand = s8.cand;
         r8.cand_cnt = s8.cand_cnt;
@@ -1048,7 +1115,7 @@ int dpq_index_search_device(dpq_index* ix, const float* d_queries, int Q, int to
             // sample (every S-th batch) -> exact re-score -> cap1 = the sample's k-th distance
             const int R = ix->opt_presample > 0 ? ix->opt_presample : (topk > 32 ? 4096 : 2048);
             if ((rc = ensure_sample_codes(ix, R))) return rc;
-            dpq::launch_presample(se.lutf, ix->d_ps_codes.as<uint8_t>(), P.cstride, P.n_local, P.M, P.K, Q, topk, R, cap0, st);
+            dpq::launch_presample(se.lutf, ix->d_ps_codes.as<uint8_t>(), P.cstride, P.n_local, P.M, P.K, Q, topk, R, cap0, ix->dead(), st);
             // The first sampled pass only has to FIND k nodes below the presample cap, not all of them: quantising
             // with levels8 * 100 / stight levels per cap while the test constant stays at levels8 accepts distances
             // up to ~stight % of cap0 -- fewer survivors to append and re-score.  A query whose sample holds fewer than
@@ -1309,6 +1376,8 @@ int64_t dpq_index_stat(dpq_index* ix, const char* name) {
     if (n == "v2_delta_nodes") return 0;  // the code-array engine has no delta records (kept for older tools)
     if (n == "device_bytes_per_node") return P.n_local > 0 ? (int64_t)((ix->ops_bytes + (P.v2 ? 0 : ix->d_codes.cap)) / (size_t)P.n_local) : 0;
     if (n == "last_fallback") return ix->last_fallback;
+    if (n == "n_deleted") return ix->n_deleted;
+    if (n == "last_delete_us") return ix->last_delete_us;
     if (n.rfind("depth_hist_", 0) == 0) {
         size_t d = (size_t)atoi(n.c_str() + 11);
         return d < P.depth_hist.size() ? P.depth_hist[d] : 0;
@@ -1344,7 +1413,7 @@ void dpq_index_close(dpq_index* ix) {
     for (DevBuf* b : {&ix->d_cap0, &ix->d_cap1, &ix->d_qlut8, &ix->d_cand8, &ix->d_cnt8, &ix->d_ovf8, &ix->d_flagged2, &ix->d_ovf, &ix->d_cand1, &ix->d_cnt1, &ix->d_part8, &ix->d_done8, &ix->d_ps_codes, &ix->d_ops, &ix->d_chunks, &ix->d_anc, &ix->d_codes, &ix->d_pos2id, &ix->d_cw,
                       &ix->d_queries, &ix->d_lutf, &ix->d_scale, &ix->d_qlut, &ix->d_cand, &ix->d_cnt,
                       &ix->d_flagged, &ix->d_ctrl, &ix->d_bound, &ix->d_key, &ix->d_fpart,
-                      &ix->d_gthr})
+                      &ix->d_gthr, &ix->d_dead, &ix->d_del_ids, &ix->d_del_tmp})
         b->release();
     if (ix->h_stage) cudaFreeHost(ix->h_stage);
     for (auto& e : ix->evs)

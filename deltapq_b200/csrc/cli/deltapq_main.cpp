@@ -156,6 +156,20 @@ static int query(const Args& a, const std::string& dataset, const std::string& e
         DPQ_TRY(dpq_index_open_file(f_tree.c_str(), nodes_arg, M, K, 0, 1, &ix));
         DPQ_TRY(dpq_index_set_codebook(ix, cb.cw.data(), cb.Ds));
     }
+    const std::string deleted = a.str("-deleted", "");
+    if (!deleted.empty()) {  // extension: vector ids (decimal, whitespace separated) that no query may return
+        std::ifstream dfs(deleted);
+        if (!dfs) return die("cannot open " + deleted);
+        std::vector<uint32_t> del;
+        unsigned long long v = 0;
+        while (dfs >> v) {
+            if (v > 0xFFFFFFFFull) return die("-deleted: id out of range in " + deleted);
+            del.push_back((uint32_t)v);
+        }
+        if (!dfs.eof()) return die("-deleted: " + deleted + " holds something other than decimal ids");
+        if (mx) DPQ_TRY(dpq_multi_delete(mx, del.data(), (int64_t)del.size()));
+        else DPQ_TRY(dpq_index_delete(ix, del.data(), (int64_t)del.size()));
+    }
     const int reps = (int)a.num("-repeat", 1);  // extension: repeat the batch (the first call pays allocations)
     double t0 = now_s();
     for (int it = 0; it < reps; ++it) {
@@ -187,7 +201,7 @@ int main(int argc, char** argv) {
     Args a{argc, argv};
     std::string dataset = a.str("-dataset", ""), ext = a.str("-ext", "fvecs"), task = a.str("-task", "approx_tree");
     int M = (int)a.num("-m", 8), K = (int)a.num("-k", 256);
-    if (dataset.empty()) return die("usage: deltapq -dataset DIR -task approx_tree|query|query_im|batch_query -m M -k K -h 1 -diff M -N N [-query_size Q] [-topk k] [-method 1|2] [-debug] [-results FILE] [-gpus N] [-parts P] [-repeat R]");
+    if (dataset.empty()) return die("usage: deltapq -dataset DIR -task approx_tree|query|query_im|batch_query -m M -k K -h 1 -diff M -N N [-query_size Q] [-topk k] [-method 1|2] [-debug] [-results FILE] [-gpus N] [-parts P] [-repeat R] [-deleted FILE]");
     if (task == "approx_tree") return approx_tree(a, dataset, M, K);
     if (task == "query" || task == "query_im" || task == "batch_query") return query(a, dataset, ext, M, K);
     return die("deltapq: task '" + task + "' is outside the B200 hot-path scope (approx_tree, query, query_im, batch_query)");

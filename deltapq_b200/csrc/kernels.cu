@@ -622,6 +622,8 @@ constexpr int FB_T = 1024;  // FB_BUF (kernels.cuh) >= FB_T + 256 (topk <= 256)
 
 // grid = (slices, query slots): block (s, y) scans slice s of the shard for the flagged queries y, y + gridDim.y, ...
 // and leaves its k best keys in part[f][s][topk]; fallback_merge_kernel sorts a query's slices together.
+// DEAD: nodes whose bit is set in a.dead are skipped.
+template <bool DEAD>
 __global__ void __launch_bounds__(FB_T) fallback_kernel(const FallbackArgs a) {
     extern __shared__ __align__(16) unsigned char fb_smem[];
     uint64_t* s_keys = reinterpret_cast<uint64_t*>(fb_smem);  // [FB_BUF]
@@ -643,7 +645,7 @@ __global__ void __launch_bounds__(FB_T) fallback_kernel(const FallbackArgs a) {
         __syncthreads();
         for (int64_t base = lo; base < hi; base += FB_T) {
             const int64_t i = base + threadIdx.x;
-            if (i < hi) {
+            if (i < hi && !(DEAD && node_dead(a.dead, (uint32_t)i))) {
                 const uint8_t* code = a.codes + (size_t)i * a.cstride;
                 const double d = exact_dist(s_lut, code, a.cstride, a.M, a.K);
                 const uint64_t key = ((uint64_t)__float_as_uint((float)d) << 32) | (uint32_t)(i + a.base_pos);
@@ -775,7 +777,7 @@ void launch_fallback(const FallbackArgs& a, cudaStream_t st) {
     const size_t sm = (size_t)FB_BUF * sizeof(uint64_t) + (size_t)a.M * a.K * sizeof(float);
     const int n_slices = fallback_slices(a.topk);
     const int qslots = a.max_flagged < 64 ? a.max_flagged : 64;
-    fallback_kernel<<<dim3((unsigned)n_slices, (unsigned)qslots), FB_T, sm, st>>>(a);
+    (a.dead ? fallback_kernel<true> : fallback_kernel<false>)<<<dim3((unsigned)n_slices, (unsigned)qslots), FB_T, sm, st>>>(a);
     fallback_merge_kernel<<<a.max_flagged < 296 ? a.max_flagged : 296, 256, 0, st>>>(a, n_slices);
 }
 

@@ -99,6 +99,12 @@ __device__ __forceinline__ void lds128_if(uint4& v, uint32_t saddr, uint32_t loa
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 __device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 
+// Deleted nodes (dpq_index_delete): one bit per local position, bit (i & 31) of word i >> 5.  A null bitmap means
+// nothing is deleted; the scan kernels then run their instantiation without any liveness test.
+__device__ __forceinline__ bool node_dead(const uint32_t* __restrict__ dead, uint32_t i) {
+    return (__ldg(dead + (i >> 5)) >> (i & 31u)) & 1u;
+}
+
 struct ScanGeom {
     int M, K, rb;      // rows = 1 << rb words per query-lane
     int pack;          // 1: one 31-bit query per lane; 2: two 15-bit queries per lane
@@ -138,7 +144,7 @@ void launch_lut_plain(const float* d_cw, int M, int K, int Ds, const float* d_qu
 cudaError_t launch_scan(const ScanArgs& a, cudaStream_t st);
 
 // ---- second-generation scan (scan2.cu) --------------------------------------------------
-struct Scan2Args {
+struct Scan2Core {
     V2Shape shape;
     const uint8_t* codes;         // [n_local][shape.nf] codes by position (8- or 16-byte aligned words)
     int64_t n_local;
@@ -152,6 +158,10 @@ struct Scan2Args {
     uint32_t* ovf;                // [n_groups*56] a candidate buffer overflowed: query needs the exact fallback
     int Q, n_groups, n_slices, n_warps;
     int kp, bcap, trigger, epoch, ramp;
+};
+// The kernel without deletions takes Scan2Core: a larger parameter block alone changed its code generation.
+struct Scan2Args : Scan2Core {
+    const uint32_t* dead;         // deleted-node bitmap by local position, or null: a deleted node is never appended
 };
 // d_qlut == nullptr: float tables only (the coarse pipeline quantises them itself)
 // d_mmax: [Q][16] floats of scratch (per-subspace table maxima; d_scale is derived from it when d_qlut is set)
@@ -198,6 +208,7 @@ struct Scan8Args {
     int thresh;                   // hit iff coarse sum < thresh (= levels + slack + 1 <= 128)
     int nf;                       // 8: narrow shape, 16: wide shape (C8Shape)
     int reuse;                    // narrow shape, 1: a strand keeps its table rows and reads only those of changed code bytes
+    const uint32_t* dead;         // deleted-node bitmap by local position, or null: a deleted node is never appended
 };
 // coarse tables: entry = min(SAT, rint(lut / unit)), unit = cap / levels, cap = the query's exact k-th
 // distance over the sample; transposed to [group][m * 256 + centroid][112 queries]
@@ -208,9 +219,10 @@ void launch_cap_from_keys(const uint64_t* d_keys, int topk, int Q, float* d_cap,
 // the presample's nodes (R evenly strided nodes of the shard, R <= 8192) gathered into a compact array [R][cstride]
 void launch_gather_sample(const uint8_t* d_codes, int cstride, int64_t n_local, int R, uint8_t* d_out, cudaStream_t st);
 // cap0[q] = exact k-th smallest distance over those R nodes (float tables, reference arithmetic): a valid,
-// loose upper bound of the true k-th distance that seeds the sample pass
+// loose upper bound of the true k-th distance that seeds the sample pass.  d_dead (may be null): deleted sample
+// nodes count as +inf, so the cap stays the k-th distance of live nodes
 void launch_presample(const float* d_lutf, const uint8_t* d_sample_codes, int cstride, int64_t n_local, int M, int K, int Q,
-                      int topk, int R, float* d_cap, cudaStream_t st);
+                      int topk, int R, float* d_cap, const uint32_t* d_dead, cudaStream_t st);
 cudaError_t launch_scan8(const Scan8Args& a, cudaStream_t st);
 struct Rescore8Args {
     const uint32_t* cand;
@@ -396,6 +408,7 @@ struct FallbackArgs {
     int M, K, topk;
     uint64_t* part;             // [max_flagged][fallback_slices(topk)][topk] per-slice results
     uint64_t* out_key;          // [Q][topk]
+    const uint32_t* dead;       // deleted-node bitmap by local position, or null
 };
 // slices of the exact fallback: as many as fit the merge buffer (slices x topk <= FB_BUF), at most 16
 inline int fallback_slices(int topk) { return topk >= 1 ? (FB_BUF / topk < 16 ? (FB_BUF / topk < 1 ? 1 : FB_BUF / topk) : 16) : 1; }
@@ -425,6 +438,7 @@ struct Scan1Args {
     uint32_t* cand_cnt;           // [Q]
     uint32_t* ovf;                // [Q]
     int ccap;
+    const uint32_t* dead;         // deleted-node bitmap by local position, or null: a deleted node is never appended
 };
 cudaError_t launch_scan1(const Scan1Args& a, cudaStream_t st);
 // exact re-score of scan1's candidate lists: one CTA per query, running top-k on (distance, position)
@@ -450,5 +464,14 @@ struct Rescore1Args {
     uint32_t* part_done;          // [Q] zeroed arrival counters (self-resetting)
 };
 void launch_rescore1(const Rescore1Args& a, cudaStream_t st);
+
+// ---- deletion (dead.cu): ids -> bits of the deleted-node bitmap ------------------------------------
+// d_ids [n_ids] sorted ascending; node i (local position) has id pos2id[i], or base_pos + i when pos2id is null.
+// set = true: sets the bit of every node whose id is listed; false: clears it.  Every 32-node word is written
+// by one thread; *d_count (zeroed by the caller) receives the number of set bits of the whole bitmap.
+void launch_mark_dead(const uint32_t* d_ids, int64_t n_ids, const uint32_t* d_pos2id, uint32_t base_pos, int64_t n_local,
+                      bool set, uint32_t* d_dead, unsigned long long* d_count, cudaStream_t st);
+// CUB radix sort of n ids (d_temp = null: *temp_bytes receives the scratch size and nothing runs)
+cudaError_t sort_ids(const uint32_t* d_in, uint32_t* d_out, int n, void* d_temp, size_t* temp_bytes, cudaStream_t st);
 
 }  // namespace dpq

@@ -22,6 +22,7 @@
 
 namespace dpq {
 int api_fail(int code, const std::string& msg);
+int api_check_device();
 }
 
 namespace {
@@ -385,6 +386,38 @@ int dpq_multi_search(dpq_multi* m, const float* queries, int Q, int topk, uint32
         if (out_id) out_id[i] = (pos < m->pos2id.size()) ? m->pos2id[pos] : pos;
     }
     return DPQ_OK;
+}
+
+// Shard and part indexes are opened without pos2id, so they take global positions: the ids are translated with
+// the QNode table first (when there is one), then every index is given the same position list and keeps its own.
+static int multi_mark_dead(dpq_multi* m, const uint32_t* ids, int64_t n, bool set, const char* what) {
+    int rc = dpq::api_check_device();
+    if (rc) return rc;
+    if (!m) return dpq::api_fail(DPQ_ERR_ARG, std::string(what) + ": null handle");
+    if (n < 0 || (n > 0 && !ids)) return dpq::api_fail(DPQ_ERR_ARG, std::string(what) + ": ids is null or n < 0");
+    if (n == 0) return DPQ_OK;
+    std::vector<uint32_t> pos;
+    const uint32_t* list = ids;
+    if (!m->pos2id.empty()) {
+        std::vector<uint32_t> sorted(ids, ids + n);
+        std::sort(sorted.begin(), sorted.end());
+        for (size_t p = 0; p < m->pos2id.size(); ++p)
+            if (std::binary_search(sorted.begin(), sorted.end(), m->pos2id[p])) pos.push_back((uint32_t)p);
+        list = pos.data();
+        n = (int64_t)pos.size();
+    }
+    for (size_t i = 0; i < m->ix.size(); ++i) {
+        CUM(cudaSetDevice(m->dev[i]));
+        rc = set ? dpq_index_delete(m->ix[i], list, n) : dpq_index_undelete(m->ix[i], list, n);
+        if (rc) return rc;
+    }
+    CUM(cudaSetDevice(0));
+    return DPQ_OK;
+}
+
+int dpq_multi_delete(dpq_multi* m, const uint32_t* ids, int64_t n) { return multi_mark_dead(m, ids, n, true, "dpq_multi_delete"); }
+int dpq_multi_undelete(dpq_multi* m, const uint32_t* ids, int64_t n) {
+    return multi_mark_dead(m, ids, n, false, "dpq_multi_undelete");
 }
 
 int64_t dpq_multi_stat(dpq_multi* m, int rank, const char* name) {

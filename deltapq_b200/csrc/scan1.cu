@@ -45,6 +45,8 @@ __device__ __forceinline__ uint32_t field_addr(uint32_t x, uint32_t base) {
     return d;
 }
 
+// DEAD: a.dead is the deleted-node bitmap; a deleted node is never appended.  DEAD = false has no test.
+template <bool DEAD>
 __global__ void __launch_bounds__(S1_T, 1) scan1_kernel(const Scan1Args a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     // table on a 16 KB boundary: address bits 6..13 are the centroid field of the lookup
@@ -124,7 +126,7 @@ __global__ void __launch_bounds__(S1_T, 1) scan1_kernel(const Scan1Args a) {
             const bool in = node < n_local;
             const bool hit0 = in && (acc & 0xFFFFu) <= thr0;
             const bool hit1 = in && live1 && (acc >> 16) <= thr1;
-            if (hit0 || hit1) {  // rare: append the position to the query's candidate list
+            if ((hit0 || hit1) && !(DEAD && node_dead(a.dead, node))) {  // rare: append the position to the query's candidate list
                 const uint32_t pos = a.base_pos + node;
                 if (hit0) {
                     const uint32_t slot = atomicAdd(&a.cand_cnt[q0], 1u);
@@ -145,9 +147,10 @@ __global__ void __launch_bounds__(S1_T, 1) scan1_kernel(const Scan1Args a) {
 
 cudaError_t launch_scan1(const Scan1Args& a, cudaStream_t st) {
     const size_t smem = (size_t)S1_TABLE + 16384;
-    cudaError_t e = cudaFuncSetAttribute(scan1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    void (*k)(const Scan1Args) = a.dead ? scan1_kernel<true> : scan1_kernel<false>;
+    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    scan1_kernel<<<(unsigned)(a.n_pairs * a.n_ranges), S1_T, smem, st>>>(a);
+    k<<<(unsigned)(a.n_pairs * a.n_ranges), S1_T, smem, st>>>(a);
     return cudaGetLastError();
 }
 

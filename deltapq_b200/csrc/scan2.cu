@@ -29,6 +29,7 @@
 #include "kernels.cuh"
 
 #include <cfloat>
+#include <type_traits>
 
 namespace dpq {
 
@@ -305,8 +306,10 @@ __device__ __noinline__ void own_compact(const Own2* o, int ql, int trigger) {
 }
 
 // NF table fields per node (= code stride), LPG active 16-byte lanes per strand, SW lanes per strand.
-template <int NF, int LPG, int SW>
-__global__ void __launch_bounds__(512, 1) scan2_kernel(const Scan2Args a) {
+// DEAD: a.dead is the deleted-node bitmap; a deleted node is never appended, so the bounds the epoch compactions
+// take from the appended candidates stay k'-th distances of live nodes.  DEAD = false is the kernel without the test.
+template <int NF, int LPG, int SW, bool DEAD>
+__global__ void __launch_bounds__(512, 1) scan2_kernel(const std::conditional_t<DEAD, Scan2Args, Scan2Core> a) {
     constexpr int QB = LPG * 8;                  // queries per CTA
     constexpr int ROWS = NF * 256;
     constexpr int ROWB = LPG * 16;               // table row bytes
@@ -446,6 +449,8 @@ __global__ void __launch_bounds__(512, 1) scan2_kernel(const Scan2Args a) {
                 bits |= (((h1 & am) >> 15 & 1u) | ((h1 & am) >> 30 & 2u)) << 2;
                 bits |= (((h2 & am) >> 15 & 1u) | ((h2 & am) >> 30 & 2u)) << 4;
                 bits |= (((h3 & am) >> 15 & 1u) | ((h3 & am) >> 30 & 2u)) << 6;
+                if constexpr (DEAD)
+                    if (bits != 0u && node_dead(a.dead, pos - a.base_pos)) bits = 0u;
                 while (bits) {
                     const int b = __ffs(bits) - 1;
                     bits &= bits - 1;
@@ -493,10 +498,19 @@ __global__ void __launch_bounds__(512, 1) scan2_kernel(const Scan2Args a) {
 cudaError_t launch_scan2(const Scan2Args& a, cudaStream_t st) {
     const size_t smem = (size_t)a.shape.lut_bytes() + MAXQB * 4 * 2 + 16;
     // 16 warps x 128 registers: more warps spill and ran 2x slower (gpurun_out/probe12.log)
-    void (*k)(const Scan2Args) = a.shape.nf == 8 ? scan2_kernel<8, 7, 8> : scan2_kernel<16, 3, 4>;
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    k<<<(unsigned)(a.n_groups * a.n_slices), (unsigned)(a.n_warps * 32), smem, st>>>(a);
+    const dim3 grid((unsigned)(a.n_groups * a.n_slices)), block((unsigned)(a.n_warps * 32));
+    cudaError_t e;
+    if (a.dead) {
+        void (*k)(const Scan2Args) = a.shape.nf == 8 ? scan2_kernel<8, 7, 8, true> : scan2_kernel<16, 3, 4, true>;
+        e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        k<<<grid, block, smem, st>>>(a);
+    } else {
+        void (*k)(const Scan2Core) = a.shape.nf == 8 ? scan2_kernel<8, 7, 8, false> : scan2_kernel<16, 3, 4, false>;
+        e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        k<<<grid, block, smem, st>>>(a);
+    }
     return cudaGetLastError();
 }
 

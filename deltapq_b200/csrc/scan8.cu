@@ -63,10 +63,11 @@ void launch_gather_sample(const uint8_t* d_codes, int cstride, int64_t n_local, 
 // it seeds the quantisation of the sample pass -- so neither the float sums nor the bucket cost exactness;
 // the kernel is instruction-issue bound (ncu: 90 % issue active), and 31 bisection rounds of shuffles and
 // barriers were most of its instructions.
-template <int PS_T>
+// DEAD: a sample node whose bit is set in `dead` counts as +inf (the cap must be the k-th distance of live nodes).
+template <int PS_T, bool DEAD>
 __global__ void __launch_bounds__(PS_T) presample_kernel(const float* __restrict__ lutf, const uint8_t* __restrict__ sample_codes, int cstride,
                                                          int64_t n_local, int M, int K, int topk, int R,
-                                                         float* __restrict__ cap) {
+                                                         float* __restrict__ cap, const uint32_t* __restrict__ dead) {
     extern __shared__ __align__(16) float s_lut[];  // M*K
     __shared__ int s_cnt[2][PS_T / 32];
     const int q = blockIdx.x;
@@ -81,7 +82,7 @@ __global__ void __launch_bounds__(PS_T) presample_kernel(const float* __restrict
     for (int t = 0; t < PER; ++t) {
         const int i = t * PS_T + threadIdx.x;
         v[t] = 0x7F800000u >> DROP;  // +inf: never counted
-        if (i < R && (int64_t)i * stride < n_local)
+        if (i < R && (int64_t)i * stride < n_local && !(DEAD && node_dead(dead, (uint32_t)((int64_t)i * stride))))
             v[t] = __float_as_uint(dist_upper_bound(s_lut, sample_codes + (size_t)i * cstride, cstride, M, K)) >> DROP;
     }
     // smallest bucket x with count(v <= x) >= topk
@@ -106,14 +107,13 @@ __global__ void __launch_bounds__(PS_T) presample_kernel(const float* __restrict
     if (threadIdx.x == 0) cap[q] = __uint_as_float((lo << DROP) | ((1u << DROP) - 1u));
 }
 void launch_presample(const float* d_lutf, const uint8_t* d_sample_codes, int cstride, int64_t n_local, int M, int K, int Q,
-                      int topk, int R, float* d_cap, cudaStream_t st) {
+                      int topk, int R, float* d_cap, const uint32_t* d_dead, cudaStream_t st) {
     // 16 values per thread: 128 threads for R <= 2048, 512 threads up to 8192
     const size_t sm = (size_t)M * K * sizeof(float);
-    if (R <= 128 * 16) {
-        presample_kernel<128><<<Q, 128, sm, st>>>(d_lutf, d_sample_codes, cstride, n_local, M, K, topk, R, d_cap);
-    } else {
-        presample_kernel<512><<<Q, 512, sm, st>>>(d_lutf, d_sample_codes, cstride, n_local, M, K, topk, R, d_cap);
-    }
+    const bool small = R <= 128 * 16;
+    auto k = small ? (d_dead ? presample_kernel<128, true> : presample_kernel<128, false>)
+                   : (d_dead ? presample_kernel<512, true> : presample_kernel<512, false>);
+    k<<<Q, small ? 128 : 512, sm, st>>>(d_lutf, d_sample_codes, cstride, n_local, M, K, topk, R, d_cap, d_dead);
 }
 
 // Coarse tables [group][m * 256 + centroid][112 queries]: NIB = false: one byte per entry (112-byte
@@ -199,7 +199,9 @@ void launch_pack8(const float* d_lutf, const float* d_cap, int M, int K, int Q, 
 //   NF = 8 : LDS.128 of the 112-byte row, word k byte b = query jj*16 + 4k + b
 //   NF = 16: LDS.64 of the 56-byte row (nibbles); sums E0, O0, E1, O1 = even / odd nibbles of the two
 //            loaded words: word w (k = w >> 1, parity p = w & 1) byte b = query jj*16 + 8k + 2b + p
-template <int NF, bool REUSE>
+// DEAD: a.dead is the deleted-node bitmap; a lane with a hit on a deleted node appends nothing.  The test sits
+// inside the rare append branch, and DEAD = false is the kernel without it.
+template <int NF, bool REUSE, bool DEAD>
 __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
     constexpr int QB = 112;                      // queries per CTA
     constexpr int ROWS = NF * 256;
@@ -327,8 +329,11 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
             const uint32_t h3 = (cmpc[3] - (d[3] & 0x7F7F7F7Fu)) & ~d[3];
             const uint32_t hit = (h0 | h1 | h2 | h3) & am;
             if (__any_sync(0xffffffffu, hit != 0u)) {
-                // rare path: one bit per byte below the bound -> append the position
-                const uint32_t hh[4] = {h0 & am, h1 & am, h2 & am, h3 & am};
+                // rare path: one bit per byte below the bound -> append the position (a deleted node: nothing)
+                uint32_t keep = am;
+                if constexpr (DEAD)
+                    if (hit != 0u && node_dead(a.dead, pos - a.base_pos)) keep = 0u;
+                const uint32_t hh[4] = {h0 & keep, h1 & keep, h2 & keep, h3 & keep};
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     uint32_t m = hh[k];
@@ -356,7 +361,9 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
 cudaError_t launch_scan8(const Scan8Args& a, cudaStream_t st) {
     const C8Shape sh = c8_shape(a.nf);
     const size_t smem = (size_t)sh.lut_bytes() + 128 * 4 + 16;
-    void (*k)(const Scan8Args) = a.nf == 16 ? scan8_kernel<16, false> : a.reuse ? scan8_kernel<8, true> : scan8_kernel<8, false>;
+    void (*k)(const Scan8Args) =
+        a.dead ? (a.nf == 16 ? scan8_kernel<16, false, true> : a.reuse ? scan8_kernel<8, true, true> : scan8_kernel<8, false, true>)
+               : (a.nf == 16 ? scan8_kernel<16, false, false> : a.reuse ? scan8_kernel<8, true, false> : scan8_kernel<8, false, false>);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     k<<<(unsigned)(a.n_groups * a.n_slices), (unsigned)(a.n_warps * 32), smem, st>>>(a);

@@ -103,6 +103,22 @@ int dpq_index_set_stream(dpq_index* idx, void* cuda_stream);
  * first-generation engine only: "pack" (1 = 31-bit, 2 = 2x15-bit filter). */
 int dpq_index_set_option(dpq_index* idx, const char* name, int64_t value);
 
+/* Deletes vectors from an open index (an extension: the reference's trees are rebuilt to drop a vector).  An id
+ * is the value this handle reports as out_id: pos2id[pos] when the index has a pos2id table, else the position
+ * (a forest part: its own vec_id, as dpq_index_open_part says).  Deletions accumulate; deleting an id twice is
+ * harmless; ids with no node in this shard are ignored, so every shard can be given the same list; n = 0 does
+ * nothing; ids == NULL with n > 0 is DPQ_ERR_ARG.  A deleted node stays in the tree as a tombstone: it is still
+ * scanned but never reported, and every search returns the top-k over the LIVE nodes with the usual rule
+ * (ascending distance, ties by lower position, the same distance bits), padded with (0xFFFFFFFF, FLT_MAX) when
+ * fewer than topk nodes are live.  The bitmap (one bit per node of the shard) appears on the first delete.
+ * dpq_index_undelete clears the same bits; once nothing is deleted the index answers exactly as one that never
+ * had deletions.  The call runs on the index's stream (the caller's after dpq_index_set_stream) and returns
+ * once the change is complete: every search issued after it sees it.  Deletions are not written to any file.
+ * The first-generation engine (DPQ_ENGINE=1) has no deletion: DPQ_ERR_ARG.  Stat "n_deleted": nodes of this
+ * shard currently deleted; "last_delete_us": host wall time of the last call. */
+int dpq_index_delete(dpq_index* idx, const uint32_t* ids, int64_t n);
+int dpq_index_undelete(dpq_index* idx, const uint32_t* ids, int64_t n);
+
 /* Replaces the per-query loop dmain:328-344 calling
  * query_processing_scan_compressed_codes_opt_o_direct (DCAT.h:2805) /
  * ..._in_memory (DCAT.h:3731): ADC table build, DeltaTree scan, top-k.
@@ -146,6 +162,11 @@ int dpq_multi_set_codebook(dpq_multi* m, const float* codewords, int Ds);
 int dpq_multi_search(dpq_multi* m, const float* queries, int Q, int topk, uint32_t* out_pos,
                      uint32_t* out_id, float* out_dist);
 int64_t dpq_multi_stat(dpq_multi* m, int rank, const char* name); /* dpq_index_stat of one shard / part */
+/* dpq_index_delete / _undelete for every shard or part.  The ids are vector ids: with a QNode file they are
+ * translated to global positions through it first; without one an id is the global position.  Every shard /
+ * part is given the same list and keeps the nodes it holds. */
+int dpq_multi_delete(dpq_multi* m, const uint32_t* ids, int64_t n);
+int dpq_multi_undelete(dpq_multi* m, const uint32_t* ids, int64_t n);
 void dpq_multi_close(dpq_multi* m);
 
 /* Raw device allocation helpers for hosts without a CUDA binding (ctypes, cgo, JNI). */
@@ -164,7 +185,8 @@ int dpq_free_host(void* hptr);
  * "timed_calls": the same summed over every search since set_option("timing_reset");
  * "last_coarse" (1 when the last search used the sample -> 8-bit coarse scan -> exact re-score
  * path), "last_latency" (1: latency mode), "last_scan8_us" / "sum_scan8_ns" (the coarse scan kernel
- * alone; in latency mode the full scan1 pass), "device_bytes_per_node", "engine". */
+ * alone; in latency mode the full scan1 pass), "device_bytes_per_node", "engine"; "n_deleted",
+ * "last_delete_us" (dpq_index_delete). */
 int64_t dpq_index_stat(dpq_index* idx, const char* name);
 
 void dpq_index_close(dpq_index* idx);
