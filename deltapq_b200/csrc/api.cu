@@ -78,7 +78,8 @@ struct dpq_index {
     int Ds = 0;
     // device-resident tree
     DevBuf d_ops, d_chunks, d_anc, d_codes, d_pos2id, d_cw, d_ovf;
-    DevBuf d_qlut8, d_cand8, d_cnt8, d_ovf8, d_flagged2, d_cap0, d_cap1, d_part8, d_done8, d_ps_codes;
+    DevBuf d_qlut8, d_cand8, d_cnt8, d_ovf8, d_flagged2, d_cap0, d_cap1, d_part8, d_done8, d_ps_codes, d_stage8;
+    int sm_slots8 = 0;  // %nsmid of the device: SM slots of the coarse scan's staging buffers (0 = not asked yet)
     int ps_R = 0;  // presample nodes currently gathered in d_ps_codes
     int last_coarse = 0;
     int last_sample_stride = 0, last_refine_stride = 0;  // strides of the sampled coarse passes of the last search
@@ -107,6 +108,7 @@ struct dpq_index {
     int opt_presample = 0;     // nodes scored exactly per query to seed the sample pass (0 auto: 2048, or 4096 for topk > 32)
     int opt_bcap8 = 0, opt_warps8 = 24, opt_levels8 = 80;  // bcap8 0 = auto (512 narrow, 2048 wide)
     int opt_reuse8 = 1;        // 1: the narrow coarse scan reads only the table rows whose code byte changed (scan8.cu); 0: all
+    int opt_stage8 = 512;      // survivor records a coarse-scan warp stages before it drains them into the lists (scan8.cu)
     int opt_stight = 100;      // percent of the presample cap the first sampled pass accepts (100 = all of it)
     int64_t opt_coarse_min = 100000;  // nodes in the shard from which the coarse search pays (gpurun_out/probe22.log)
     int opt_dbg_bound = 0x8000;  // developer probe: initial exclusive bound (results are wrong below 0x8000)
@@ -593,6 +595,7 @@ int dpq_index_set_option(dpq_index* ix, const char* name, int64_t v) {
     else if (n == "bcap8") ix->opt_bcap8 = v <= 0 ? 0 : std::max(32, (int)v);
     else if (n == "warps8") ix->opt_warps8 = std::max(2, std::min(24, (int)v));
     else if (n == "reuse8") ix->opt_reuse8 = v != 0;
+    else if (n == "stage8") ix->opt_stage8 = std::max(32, std::min(1 << 16, (int)v));
     else if (n == "coarse_min") ix->opt_coarse_min = v;
     else if (n == "seed") ix->opt_seed = (int)v;
     else if (n == "refine") ix->opt_refine = (int)v;
@@ -944,6 +947,8 @@ int dpq_index_search_device(dpq_index* ix, const float* d_queries, int Q, int to
         if ((rc = ix->d_cnt8.ensure(items8 * c8.qb * 4))) return rc;
         if ((rc = ix->d_ovf8.ensure((size_t)g8_groups * c8.qb * 4))) return rc;
         if ((rc = ix->d_flagged2.ensure((size_t)max_flagged * 4))) return rc;
+        if (!ix->sm_slots8) CU(dpq::scan8_sm_slots(ix->d_flagged2.as<int>(), &ix->sm_slots8, ix->stream));
+        if ((rc = ix->d_stage8.ensure((size_t)ix->sm_slots8 * 24 * ix->opt_stage8 * 8))) return rc;
         if (r8_parts > 1) {
             if ((rc = ix->d_part8.ensure((size_t)Q * r8_parts * topk * 8))) return rc;
             const bool fresh = ix->d_done8.cap < (size_t)Q * 4;
@@ -1091,6 +1096,8 @@ int dpq_index_search_device(dpq_index* ix, const float* d_queries, int Q, int to
         s8.nf = c8.nf;
         s8.reuse = ix->opt_reuse8;
         s8.dead = ix->dead();
+        s8.stage = ix->d_stage8.as<uint2>();
+        s8.stage_cap = ix->opt_stage8;
         dpq::Rescore8Args r8;
         r8.cand = s8.cand;
         r8.cand_cnt = s8.cand_cnt;
@@ -1410,7 +1417,7 @@ void dpq_index_close(dpq_index* ix) {
     if (!ix) return;
     cudaSetDevice(ix->device);
     if (ix->stream) cudaStreamSynchronize(ix->stream);
-    for (DevBuf* b : {&ix->d_cap0, &ix->d_cap1, &ix->d_qlut8, &ix->d_cand8, &ix->d_cnt8, &ix->d_ovf8, &ix->d_flagged2, &ix->d_ovf, &ix->d_cand1, &ix->d_cnt1, &ix->d_part8, &ix->d_done8, &ix->d_ps_codes, &ix->d_ops, &ix->d_chunks, &ix->d_anc, &ix->d_codes, &ix->d_pos2id, &ix->d_cw,
+    for (DevBuf* b : {&ix->d_cap0, &ix->d_cap1, &ix->d_qlut8, &ix->d_cand8, &ix->d_cnt8, &ix->d_ovf8, &ix->d_flagged2, &ix->d_ovf, &ix->d_cand1, &ix->d_cnt1, &ix->d_part8, &ix->d_done8, &ix->d_ps_codes, &ix->d_stage8, &ix->d_ops, &ix->d_chunks, &ix->d_anc, &ix->d_codes, &ix->d_pos2id, &ix->d_cw,
                       &ix->d_queries, &ix->d_lutf, &ix->d_scale, &ix->d_qlut, &ix->d_cand, &ix->d_cnt,
                       &ix->d_flagged, &ix->d_ctrl, &ix->d_bound, &ix->d_key, &ix->d_fpart,
                       &ix->d_gthr, &ix->d_dead, &ix->d_del_ids, &ix->d_del_tmp})

@@ -209,6 +209,8 @@ struct Scan8Args {
     int nf;                       // 8: narrow shape, 16: wide shape (C8Shape)
     int reuse;                    // narrow shape, 1: a strand keeps its table rows and reads only those of changed code bytes
     const uint32_t* dead;         // deleted-node bitmap by local position, or null: a deleted node is never appended
+    uint2* stage;                 // [SM slots][24 warps][stage_cap] survivor records (one resident CTA per SM)
+    int stage_cap;                // records per warp, >= 32: how often a warp drains, never what it finds
 };
 // coarse tables: entry = min(SAT, rint(lut / unit)), unit = cap / levels, cap = the query's exact k-th
 // distance over the sample; transposed to [group][m * 256 + centroid][112 queries]
@@ -224,6 +226,8 @@ void launch_gather_sample(const uint8_t* d_codes, int cstride, int64_t n_local, 
 void launch_presample(const float* d_lutf, const uint8_t* d_sample_codes, int cstride, int64_t n_local, int M, int K, int Q,
                       int topk, int R, float* d_cap, const uint32_t* d_dead, cudaStream_t st);
 cudaError_t launch_scan8(const Scan8Args& a, cudaStream_t st);
+// number of %smid values of the device (the SM slots of Scan8Args::stage); d_tmp: one device int; syncs st
+cudaError_t scan8_sm_slots(int* d_tmp, int* n_slots, cudaStream_t st);
 struct Rescore8Args {
     const uint32_t* cand;
     const uint32_t* cand_cnt;

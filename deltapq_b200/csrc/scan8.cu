@@ -23,7 +23,7 @@
 // overflows flags its query for the exact fallback.  No result ever depends on the coarse values.
 //
 // The kernels are scan2's strand design (one code word per node, four nodes per warp step) with the
-// candidate machinery reduced to an append: the bound is the same constant for every query, so
+// candidate machinery reduced to a staged append: the bound is the same constant for every query, so
 // there are no epochs, barriers or compactions.
 #include "kernels.cuh"
 
@@ -199,8 +199,51 @@ void launch_pack8(const float* d_lutf, const float* d_cap, int M, int K, int Q, 
 //   NF = 8 : LDS.128 of the 112-byte row, word k byte b = query jj*16 + 4k + b
 //   NF = 16: LDS.64 of the 56-byte row (nibbles); sums E0, O0, E1, O1 = even / odd nibbles of the two
 //            loaded words: word w (k = w >> 1, parity p = w & 1) byte b = query jj*16 + 8k + 2b + p
-// DEAD: a.dead is the deleted-node bitmap; a lane with a hit on a deleted node appends nothing.  The test sits
-// inside the rare append branch, and DEAD = false is the kernel without it.
+//
+// Survivors are staged, not appended in the node loop.  A lane whose node passes for any of its 16
+// queries writes one 8-byte record {position, jj << 4 | hit bits} to its warp's staging buffer in
+// global memory; the slot is a warp-uniform counter plus the lane's rank in the step's ballot, so a
+// step with hits has no atomics, no divergent loops and nothing that waits on a returned value.  The per-hit
+// atomicAdd + store it replaces held most of the kernel's instructions and stall samples on the
+// steps that took it (DESIGN.md section 8).  The warp expands its records into the per-(item, query)
+// lists (drain8) whenever the next step could overflow its buffer and once at the end: the lists,
+// their counts (clipped at bcap) and the overflow flags are exactly those of an in-loop append, in
+// another order within a list, which nothing downstream depends on.  The staging capacity changes
+// only how often a warp drains.  A buffer belongs to (SM, warp): one CTA per SM (checked at launch).
+// DEAD: a.dead is the deleted-node bitmap; a lane whose node is deleted stages nothing.  The test
+// sits inside the rare branch (one bitmap word per lane with a hit), before the ballot: testing in the
+// drain instead stages every deleted node that passes, and with most of the tree deleted the loose
+// cap of the live nodes passes many (25 % slower at 99 % deleted).  DEAD = false is the kernel without it.
+template <int NF>
+__device__ __forceinline__ void drain8(const uint2* __restrict__ rec, int n, uint32_t* s_cnt, uint32_t* __restrict__ my_cand,
+                                    const Scan8Args& a, int grp, int lane) {
+    constexpr int QB = 112;
+    __syncwarp();  // the warp's records are visible to all of its lanes
+    for (int i0 = 0; i0 < n; i0 += 32) {  // warp-uniform loops: the node loop stays convergent
+        uint32_t m = 0u, pos = 0u;
+        int jj = 0;
+        if (i0 + lane < n) {
+            const uint2 r = __ldcg(rec + i0 + lane);
+            m = r.y & 0x0F0F0F0Fu;  // bit 8 b + k: byte b of word k
+            jj = (int)(r.y >> 4) & 7;
+            pos = r.x;
+        }
+        while (__any_sync(0xffffffffu, m != 0u)) {
+            if (m) {
+                const int bit = __ffs(m) - 1;
+                m &= m - 1;
+                const int b = bit >> 3, k = bit & 3;
+                const int q = NF == 8 ? 4 * k + b : 8 * (k >> 1) + 2 * b + (k & 1);
+                const int ql = jj * 16 + q;
+                const uint32_t slot = atomicAdd(&s_cnt[ql], 1u);
+                if (slot < (uint32_t)a.bcap) __stcg(my_cand + (size_t)ql * a.bcap + slot, pos);
+                else a.ovf[(size_t)grp * QB + ql] = 1u;
+            }
+        }
+    }
+    __syncwarp();  // every record is read before the buffer is refilled
+}
+
 template <int NF, bool REUSE, bool DEAD>
 __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
     constexpr int QB = 112;                      // queries per CTA
@@ -272,6 +315,66 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
 #pragma unroll
     for (int r = 0; r < 8; ++r) A[r] = make_uint4(0u, 0u, 0u, 0u);
 
+    // this warp's staging buffer: [SM][24 warps][stage_cap] records
+    uint32_t smid;
+    asm("mov.u32 %0, %%smid;" : "=r"(smid));
+    uint2* stage = a.stage + ((size_t)smid * 24 + (size_t)warp) * (size_t)a.stage_cap;
+    const uint32_t lt_mask = (1u << lane) - 1u;
+    const uint32_t jj_tag = (uint32_t)jj << 4;
+    int n_staged = 0;  // warp-uniform
+
+    // One node of a strand: its M rows (NF = 8: those whose code byte changed, REUSE), the byte sums, the
+    // SWAR hit test, and on a hit one staged record.  ok: the node exists.
+    auto node = [&](const CodeT w, const uint2 chg, const bool ok, const uint32_t p) {
+        uint32_t d[4];
+        if constexpr (NF == 8) {
+            const uint32_t w2[2] = {w.x, w.y};
+            const uint32_t ch2[2] = {REUSE ? chg.x : ~0u, REUSE ? chg.y : ~0u};
+#pragma unroll
+            for (int r = 0; r < 8; ++r)
+                lds128_if(A[r], rowaddr<ROWB>(lut_base, w2[r >> 2], r & 3) + (uint32_t)(r * SUB), ch2[r >> 2] & (0xFFu << (8 * (r & 3))));
+            d[0] = (A[0].x + A[1].x + A[2].x) + (A[3].x + A[4].x + A[5].x) + (A[6].x + A[7].x);
+            d[1] = (A[0].y + A[1].y + A[2].y) + (A[3].y + A[4].y + A[5].y) + (A[6].y + A[7].y);
+            d[2] = (A[0].z + A[1].z + A[2].z) + (A[3].z + A[4].z + A[5].z) + (A[6].z + A[7].z);
+            d[3] = (A[0].w + A[1].w + A[2].w) + (A[3].w + A[4].w + A[5].w) + (A[6].w + A[7].w);
+        } else {
+            const uint32_t w4[4] = {w.x, w.y, w.z, w.w};
+            d[0] = d[1] = d[2] = d[3] = 0u;
+#pragma unroll
+            for (int h = 0; h < 4; ++h) {  // four rows at a time: four 64-bit reads in flight per step
+                const uint2 A0 = lds64(rowaddr<ROWB>(lut_base, w4[h], 0) + (uint32_t)((4 * h + 0) * SUB));
+                const uint2 A1 = lds64(rowaddr<ROWB>(lut_base, w4[h], 1) + (uint32_t)((4 * h + 1) * SUB));
+                const uint2 A2 = lds64(rowaddr<ROWB>(lut_base, w4[h], 2) + (uint32_t)((4 * h + 2) * SUB));
+                const uint2 A3 = lds64(rowaddr<ROWB>(lut_base, w4[h], 3) + (uint32_t)((4 * h + 3) * SUB));
+                constexpr uint32_t LO = 0x0F0F0F0Fu;
+                d[0] += ((A0.x & LO) + (A1.x & LO)) + ((A2.x & LO) + (A3.x & LO));
+                d[1] += (((A0.x >> 4) & LO) + ((A1.x >> 4) & LO)) + (((A2.x >> 4) & LO) + ((A3.x >> 4) & LO));
+                d[2] += ((A0.y & LO) + (A1.y & LO)) + ((A2.y & LO) + (A3.y & LO));
+                d[3] += (((A0.y >> 4) & LO) + ((A1.y >> 4) & LO)) + (((A2.y >> 4) & LO) + ((A3.y >> 4) & LO));
+            }
+        }
+        const uint32_t am = ok ? 0x80808080u : 0u;
+        const uint32_t h0 = (cmpc[0] - (d[0] & 0x7F7F7F7Fu)) & ~d[0];
+        const uint32_t h1 = (cmpc[1] - (d[1] & 0x7F7F7F7Fu)) & ~d[1];
+        const uint32_t h2 = (cmpc[2] - (d[2] & 0x7F7F7F7Fu)) & ~d[2];
+        const uint32_t h3 = (cmpc[3] - (d[3] & 0x7F7F7F7Fu)) & ~d[3];
+        uint32_t hit = (h0 | h1 | h2 | h3) & am;
+        if (__any_sync(0xffffffffu, hit != 0u)) {  // the ballot and the fold stay off the common path
+            // a deleted node stages nothing: under a heavily deleted tree most nodes that pass are deleted
+            if constexpr (DEAD)
+                if (hit != 0u && node_dead(a.dead, p - a.base_pos)) hit = 0u;
+            const uint32_t bal = __ballot_sync(0xffffffffu, hit != 0u);
+            // bit 8 b + k of the fold: byte b of word k is below the bound
+            const uint32_t hb = (((h0 & am) >> 7) | ((h1 & am) >> 6)) | (((h2 & am) >> 5) | ((h3 & am) >> 4));
+            if (hit) __stcg(stage + n_staged + __popc(bal & lt_mask), make_uint2(p, hb | jj_tag));
+            n_staged += __popc(bal);
+            if (n_staged > a.stage_cap - 32) {  // a step stages at most 28 records
+                drain8<NF>(stage, n_staged, s_cnt, my_cand, a, grp, lane);
+                n_staged = 0;
+            }
+        }
+    };
+
     for (int round = 0; round < n_rounds; ++round) {
         const int bt = b_lo + round * a.n_warps + warp;
         const int c = bt * a.bt_stride * SPW + strand;
@@ -282,80 +385,66 @@ __global__ void __launch_bounds__(768, 1) scan8_kernel(const Scan8Args a) {
             n_nodes = (int)min((int64_t)C, a.n_local - (int64_t)nix);
             pos = a.base_pos + nix;
         }
-        CodeT rec = CodeWord<NF>::zero(), nxt;
-        if (n_nodes > 0) rec = __ldg(codes + nix);
         // code bytes that differ from the strand's previous node: at a chunk start all of them, on an
         // idle strand none (past a chunk's last node the code is 0: one read of the changed rows, then none)
         uint2 chg = n_nodes > 0 ? make_uint2(~0u, ~0u) : make_uint2(0u, 0u);
+        if constexpr (NF == 8) {
+            // Two nodes' code words per 128-bit load (C is even, so a pair never straddles 16 bytes): half
+            // the load wavefronts of one LDG.64 per node, double-buffered one pair ahead.
+            const uint4* pairs = reinterpret_cast<const uint4*>(codes);
+            auto load_pair = [&](uint32_t at, int first) {  // nodes `first`, `first` + 1 of the chunk
+                uint4 v = make_uint4(0u, 0u, 0u, 0u);
+                if (first + 1 < n_nodes) v = __ldg(pairs + (at >> 1));
+                else if (first < n_nodes) { const uint2 h = __ldg(codes + at); v.x = h.x; v.y = h.y; }
+                return v;
+            };
+            uint4 cur = load_pair(nix, 0);
 #pragma unroll 1
-        for (int it = 0; it < C; ++it) {
-            ++nix;
-            if ((it & (PF - 1)) == 0) {  // warp-uniform: one L2 prefetch per 128-byte line of codes, three lines ahead
-                if (it + 3 * PF + 1 < n_nodes) prefetch_l2(codes + nix + 3 * PF);
-            }
-            nxt = CodeWord<NF>::zero();
-            if (it + 1 < n_nodes) nxt = __ldg(codes + nix);
-            uint32_t d[4];
-            if constexpr (NF == 8) {
-                const uint32_t w2[2] = {rec.x, rec.y};
-                const uint32_t ch2[2] = {REUSE ? chg.x : ~0u, REUSE ? chg.y : ~0u};
-#pragma unroll
-                for (int r = 0; r < 8; ++r)
-                    lds128_if(A[r], rowaddr<ROWB>(lut_base, w2[r >> 2], r & 3) + (uint32_t)(r * SUB), ch2[r >> 2] & (0xFFu << (8 * (r & 3))));
-                d[0] = (A[0].x + A[1].x + A[2].x) + (A[3].x + A[4].x + A[5].x) + (A[6].x + A[7].x);
-                d[1] = (A[0].y + A[1].y + A[2].y) + (A[3].y + A[4].y + A[5].y) + (A[6].y + A[7].y);
-                d[2] = (A[0].z + A[1].z + A[2].z) + (A[3].z + A[4].z + A[5].z) + (A[6].z + A[7].z);
-                d[3] = (A[0].w + A[1].w + A[2].w) + (A[3].w + A[4].w + A[5].w) + (A[6].w + A[7].w);
-            } else {
-                const uint32_t w4[4] = {rec.x, rec.y, rec.z, rec.w};
-                d[0] = d[1] = d[2] = d[3] = 0u;
-#pragma unroll
-                for (int h = 0; h < 4; ++h) {  // four rows at a time: four 64-bit reads in flight per step
-                    const uint2 A0 = lds64(rowaddr<ROWB>(lut_base, w4[h], 0) + (uint32_t)((4 * h + 0) * SUB));
-                    const uint2 A1 = lds64(rowaddr<ROWB>(lut_base, w4[h], 1) + (uint32_t)((4 * h + 1) * SUB));
-                    const uint2 A2 = lds64(rowaddr<ROWB>(lut_base, w4[h], 2) + (uint32_t)((4 * h + 2) * SUB));
-                    const uint2 A3 = lds64(rowaddr<ROWB>(lut_base, w4[h], 3) + (uint32_t)((4 * h + 3) * SUB));
-                    constexpr uint32_t LO = 0x0F0F0F0Fu;
-                    d[0] += ((A0.x & LO) + (A1.x & LO)) + ((A2.x & LO) + (A3.x & LO));
-                    d[1] += (((A0.x >> 4) & LO) + ((A1.x >> 4) & LO)) + (((A2.x >> 4) & LO) + ((A3.x >> 4) & LO));
-                    d[2] += ((A0.y & LO) + (A1.y & LO)) + ((A2.y & LO) + (A3.y & LO));
-                    d[3] += (((A0.y >> 4) & LO) + ((A1.y >> 4) & LO)) + (((A2.y >> 4) & LO) + ((A3.y >> 4) & LO));
+            for (int it = 0; it < C; it += 2) {
+                nix += 2;
+                if ((it & (PF - 1)) == 0) {  // warp-uniform: one L2 prefetch per 128-byte line of codes, three lines ahead
+                    if (it + 3 * PF + 1 < n_nodes) prefetch_l2(codes + nix - 1 + 3 * PF);
                 }
+                const uint4 nxt = load_pair(nix, it + 2);
+                node(make_uint2(cur.x, cur.y), chg, it < n_nodes, pos);
+                node(make_uint2(cur.z, cur.w), make_uint2(cur.z ^ cur.x, cur.w ^ cur.y), it + 1 < n_nodes, pos + 1u);
+                chg = make_uint2(nxt.x ^ cur.z, nxt.y ^ cur.w);
+                cur = nxt;
+                pos += 2u;
             }
-            const uint32_t am = it < n_nodes ? 0x80808080u : 0u;
-            const uint32_t h0 = (cmpc[0] - (d[0] & 0x7F7F7F7Fu)) & ~d[0];
-            const uint32_t h1 = (cmpc[1] - (d[1] & 0x7F7F7F7Fu)) & ~d[1];
-            const uint32_t h2 = (cmpc[2] - (d[2] & 0x7F7F7F7Fu)) & ~d[2];
-            const uint32_t h3 = (cmpc[3] - (d[3] & 0x7F7F7F7Fu)) & ~d[3];
-            const uint32_t hit = (h0 | h1 | h2 | h3) & am;
-            if (__any_sync(0xffffffffu, hit != 0u)) {
-                // rare path: one bit per byte below the bound -> append the position (a deleted node: nothing)
-                uint32_t keep = am;
-                if constexpr (DEAD)
-                    if (hit != 0u && node_dead(a.dead, pos - a.base_pos)) keep = 0u;
-                const uint32_t hh[4] = {h0 & keep, h1 & keep, h2 & keep, h3 & keep};
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    uint32_t m = hh[k];
-                    while (m) {
-                        const int b = (__ffs(m) - 1) >> 3;
-                        m &= m - 1;
-                        const int r = NF == 8 ? 4 * k + b : 8 * (k >> 1) + 2 * b + (k & 1);
-                        const int ql = jj * 16 + r;
-                        const uint32_t slot = atomicAdd(&s_cnt[ql], 1u);
-                        if (slot < (uint32_t)a.bcap) __stcg(my_cand + (size_t)ql * a.bcap + slot, pos);
-                        else a.ovf[(size_t)grp * QB + ql] = 1u;
-                    }
+        } else {
+            CodeT rec = CodeWord<NF>::zero(), nxt;
+            if (n_nodes > 0) rec = __ldg(codes + nix);
+#pragma unroll 1
+            for (int it = 0; it < C; ++it) {
+                ++nix;
+                if ((it & (PF - 1)) == 0) {  // warp-uniform: one L2 prefetch per 128-byte line of codes, three lines ahead
+                    if (it + 3 * PF + 1 < n_nodes) prefetch_l2(codes + nix + 3 * PF);
                 }
+                nxt = CodeWord<NF>::zero();
+                if (it + 1 < n_nodes) nxt = __ldg(codes + nix);
+                node(rec, chg, it < n_nodes, pos);
+                rec = nxt;
+                ++pos;
             }
-            if constexpr (REUSE) chg = make_uint2(nxt.x ^ rec.x, nxt.y ^ rec.y);
-            rec = nxt;
-            ++pos;
         }
     }
+    if (n_staged) drain8<NF>(stage, n_staged, s_cnt, my_cand, a, grp, lane);
     __syncthreads();
     for (int ql = threadIdx.x; ql < QB; ql += blockDim.x)
         a.cand_cnt[(size_t)item * QB + ql] = min(s_cnt[ql], (uint32_t)a.bcap);
+}
+
+__global__ void nsmid_kernel(int* out) {
+    uint32_t n;
+    asm("mov.u32 %0, %%nsmid;" : "=r"(n));
+    *out = (int)n;
+}
+cudaError_t scan8_sm_slots(int* d_tmp, int* n_slots, cudaStream_t st) {
+    nsmid_kernel<<<1, 1, 0, st>>>(d_tmp);
+    cudaError_t e = cudaMemcpyAsync(n_slots, d_tmp, sizeof(int), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    return e;
 }
 
 cudaError_t launch_scan8(const Scan8Args& a, cudaStream_t st) {
@@ -366,6 +455,11 @@ cudaError_t launch_scan8(const Scan8Args& a, cudaStream_t st) {
                : (a.nf == 16 ? scan8_kernel<16, false, false> : a.reuse ? scan8_kernel<8, true, false> : scan8_kernel<8, false, false>);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
+    // the staging buffers are indexed by SM: a second resident CTA would share them
+    int per_sm = 0;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, a.n_warps * 32, smem);
+    if (e != cudaSuccess) return e;
+    if (per_sm > 1 || a.n_warps > 24 || a.stage_cap < 32 || !a.stage || (a.chunk_nodes & 1)) return cudaErrorInvalidConfiguration;
     k<<<(unsigned)(a.n_groups * a.n_slices), (unsigned)(a.n_warps * 32), smem, st>>>(a);
     return cudaGetLastError();
 }
