@@ -27,6 +27,7 @@ SYMBOLS = [
     "dpq_program_free", "dpq_tree_build", "dpq_tree_from_edges", "dpq_tree_size", "dpq_tree_copy",
     "dpq_tree_free", "dpq_multi_open_file", "dpq_multi_set_codebook", "dpq_multi_search", "dpq_multi_stat",
     "dpq_multi_close", "dpq_index_delete", "dpq_index_undelete", "dpq_multi_delete", "dpq_multi_undelete",
+    "dpq_index_add", "dpq_index_add_vectors", "dpq_multi_add", "dpq_multi_add_vectors",
 ]
 
 
@@ -110,6 +111,10 @@ def lib():
     L.dpq_multi_close.restype = None
     for name in ("dpq_index_delete", "dpq_index_undelete", "dpq_multi_delete", "dpq_multi_undelete"):
         getattr(L, name).argtypes = [vp, vp, i64]
+    for name in ("dpq_index_add", "dpq_multi_add"):
+        getattr(L, name).argtypes = [vp, vp, i64, vp, vp]
+    for name in ("dpq_index_add_vectors", "dpq_multi_add_vectors"):
+        getattr(L, name).argtypes = [vp, vp, i64, i32, vp, vp]
     _lib = L
     return L
 
@@ -176,6 +181,27 @@ _PINNED = []
 def _id_array(ids):
     ids = np.ascontiguousarray(np.asarray(ids).reshape(-1), np.uint32)
     return ids, (_ptr(ids) if ids.size else None)
+
+
+def _add(fn, h, data, ids, D=None):
+    """dpq_index_add / dpq_multi_add (D None: data are codes [n][M] uint8) or their _add_vectors forms (data
+    [n][D] float32) -> the position given to each input row."""
+    if D is None:
+        data = np.ascontiguousarray(data, np.uint8)
+    else:
+        data = np.ascontiguousarray(data, np.float32)
+    n = data.shape[0]
+    p_ids = None
+    if ids is not None:
+        ids = np.ascontiguousarray(np.asarray(ids).reshape(-1), np.uint32)
+        assert ids.size == n
+        p_ids = _ptr(ids)
+    pos = np.empty(n, np.uint32)
+    if D is None:
+        _check(fn(h, _ptr(data), n, p_ids, _ptr(pos)))
+    else:
+        _check(fn(h, _ptr(data), n, data.shape[1], p_ids, _ptr(pos)))
+    return pos
 
 
 def unpack_keys(keys):
@@ -255,6 +281,14 @@ class DeltaTreeIndex:
         ids, p = _id_array(ids)
         _check(lib().dpq_index_undelete(self._h, p, ids.size))
 
+    def add(self, codes, ids=None):
+        """dpq_index_add: codes [n][M] appended (ids None: id = position); returns each row's position."""
+        return _add(lib().dpq_index_add, self._h, codes, ids)
+
+    def add_vectors(self, x, ids=None):
+        """dpq_index_add_vectors: x [n][D] encoded with the index's codebook and appended; returns the positions."""
+        return _add(lib().dpq_index_add_vectors, self._h, x, ids, D=np.asarray(x).shape[1])
+
     def search_device(self, d_queries_ptr, Q, topk, d_out_ptr):
         _check(lib().dpq_index_search_device(self._h, d_queries_ptr, Q, topk, d_out_ptr))
 
@@ -308,6 +342,13 @@ class MultiIndex:
     def undelete(self, ids):
         ids, p = _id_array(ids)
         _check(lib().dpq_multi_undelete(self._h, p, ids.size))
+
+    def add(self, codes, ids=None):
+        """dpq_multi_add: appended to the index that ends the position space; returns the global positions."""
+        return _add(lib().dpq_multi_add, self._h, codes, ids)
+
+    def add_vectors(self, x, ids=None):
+        return _add(lib().dpq_multi_add_vectors, self._h, x, ids, D=np.asarray(x).shape[1])
 
     def stat(self, rank, name):
         return int(lib().dpq_multi_stat(self._h, rank, name.encode()))

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "../../include/dpq.h"
+#include "encode_tc.cuh"
 #include "kernels.cuh"
 #include "tree_internal.h"
 
@@ -37,7 +38,7 @@ int check_device();
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
-    int ensure(size_t bytes) {
+    int ensure(size_t bytes) {  // drops the contents when it reallocates
         if (bytes <= cap) return DPQ_OK;
         if (p) cudaFree(p);
         p = nullptr;
@@ -61,6 +62,23 @@ struct DevBuf {
         return reinterpret_cast<T*>(p);
     }
 };
+
+// A scratch buffer released on every return path (DevBuf itself has none: index members outlive calls).
+struct Scratch {
+    DevBuf b;
+    ~Scratch() { b.release(); }
+};
+
+// True when p is device memory of `device`, which an index's kernels may read directly.  Host memory and memory of
+// another device (no peer access is enabled) are copied to the index's device first, with cudaMemcpyDefault.
+bool on_device(const void* p, int device) {
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+        (void)cudaGetLastError();
+        return false;
+    }
+    return at.type == cudaMemoryTypeDevice && at.device == device;
+}
 
 }  // namespace
 
@@ -127,6 +145,11 @@ struct dpq_index {
     int64_t n_deleted = 0;
     int64_t last_delete_us = 0;  // host wall clock of the last dpq_index_delete / _undelete (ends in a stream sync)
     const uint32_t* dead() const { return d_dead.p ? d_dead.as<uint32_t>() : nullptr; }
+    // appended nodes (dpq_index_add): only the index whose positions end the position space accepts them
+    bool ends_range = true;    // false for shards rank < n_ranks - 1
+    int opt_add_order = 1;     // 1: an add batch is laid out sorted by code word; 0: in input order
+    int64_t n_added = 0;
+    int64_t last_add_us = 0;   // host wall clock of the last dpq_index_add / _add_vectors (ends in a stream sync)
 };
 
 namespace {
@@ -219,6 +242,31 @@ int upload(DevBuf& b, const void* src, size_t bytes, cudaStream_t st) {
     int rc = b.ensure(std::max<size_t>(bytes, 16));
     if (rc) return rc;
     if (bytes) CU(cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, st));
+    return DPQ_OK;
+}
+
+// Keeps the first `used` bytes of b and makes room for `need`: a new block of at least 1.5x the old capacity (many
+// small adds stay amortised), the contents copied device to device on st, every byte past `used` zeroed, then the
+// old block freed.
+int grow(DevBuf& b, size_t used, size_t need, cudaStream_t st) {
+    if (need <= b.cap) return DPQ_OK;
+    const size_t want = std::max(need, b.cap + b.cap / 2) + 256;
+    void* p = nullptr;
+    cudaError_t e = cudaMalloc(&p, want);
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();
+        return fail(DPQ_ERR_NOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+    }
+    if (used) e = cudaMemcpyAsync(p, b.p, used, cudaMemcpyDeviceToDevice, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(static_cast<char*>(p) + used, 0, want - used, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // searches still in flight read the old block
+    if (e != cudaSuccess) {
+        cudaFree(p);
+        return fail(DPQ_ERR_CUDA, std::string("growing a device buffer: ") + cudaGetErrorString(e));
+    }
+    b.release();
+    b.p = p;
+    b.cap = want;
     return DPQ_OK;
 }
 
@@ -324,6 +372,7 @@ static int open_common(const uint8_t* payload, int64_t n_bytes, int64_t n_codes,
         delete ix;
         return fail(DPQ_ERR_FORMAT, "dpq_index_open: " + err);
     }
+    ix->ends_range = rank == n_ranks - 1;
     if (first_pos) {  // one tree of a forest: every position this index reports is shifted
         ix->pos_shift = first_pos;
         ix->prog.base_pos += first_pos;
@@ -493,6 +542,7 @@ static int open_tree_shard_impl(dpq_tree* t, int rank, int n_ranks, int64_t firs
     if (hi == lo) lo = hi = n;  // an empty shard reports base_pos = n_codes like the stream reader (program.cpp)
     dpq_index* ix = new dpq_index();
     ix->device = g_device;
+    ix->ends_range = rank == n_ranks - 1;
     dpq::ScanProgram& P = ix->prog;
     P.M = M;
     P.K = K;
@@ -605,6 +655,7 @@ int dpq_index_set_option(dpq_index* ix, const char* name, int64_t v) {
     else if (n == "presample") ix->opt_presample = v <= 0 ? 0 : std::max(64, std::min(8192, (int)v));
     else if (n == "levels8") ix->opt_levels8 = std::max(31, std::min(123, (int)v));
     else if (n == "stight") ix->opt_stight = std::max(50, std::min(100, (int)v));
+    else if (n == "add_order") ix->opt_add_order = v != 0;
     else return fail(DPQ_ERR_ARG, "unknown option " + n);
     return DPQ_OK;
 }
@@ -664,6 +715,161 @@ static int mark_dead(dpq_index* ix, const uint32_t* ids, int64_t n, bool set, co
 
 int dpq_index_delete(dpq_index* ix, const uint32_t* ids, int64_t n) { return mark_dead(ix, ids, n, true, "dpq_index_delete"); }
 int dpq_index_undelete(dpq_index* ix, const uint32_t* ids, int64_t n) { return mark_dead(ix, ids, n, false, "dpq_index_undelete"); }
+
+// dpq_index_add / dpq_index_add_vectors: the checks both share.  *done = true when there is nothing to do.
+static int add_check(dpq_index* ix, const void* data, int64_t n, const char* what, bool* done) {
+    *done = true;
+    int rc = check_device();
+    if (rc) return rc;
+    if (!ix) return fail(DPQ_ERR_ARG, std::string(what) + ": null index");
+    if (n < 0 || (n > 0 && !data)) return fail(DPQ_ERR_ARG, std::string(what) + ": input is null or n < 0");
+    if (n > 0x7FFFFFFFLL) return fail(DPQ_ERR_ARG, std::string(what) + ": more than 2^31 - 1 rows in one call");
+    const dpq::ScanProgram& P = ix->prog;
+    if (!P.v2)
+        return fail(DPQ_ERR_ARG, std::string(what) +
+                                     ": adding needs the code-array engine (this index runs the first-generation engine, DPQ_ENGINE=1)");
+    if (!ix->ends_range)
+        return fail(DPQ_ERR_ARG, std::string(what) + ": only the last shard (or a whole tree, or a forest part) accepts adds");
+    if (P.base_pos + P.n_local + n > 0xFFFFFFFFLL)
+        return fail(DPQ_ERR_ARG, std::string(what) + ": an appended position would reach 0xFFFFFFFF");
+    if (n == 0) {
+        ix->last_add_us = 0;
+        return DPQ_OK;
+    }
+    *done = false;
+    return DPQ_OK;
+}
+
+// Appends n nodes whose codes d_in [n][M] are on the device: sorted by code word on the device (add.cu) unless
+// add_order = 0, then the padded words go to the tail of d_codes, the ids to the tail of the id table and the
+// positions to out_pos.  ids / out_pos may be host or device pointers.  Host state changes only once the device
+// work has completed, so a failed call leaves the index as it was.
+static int append_nodes(dpq_index* ix, const uint8_t* d_in, int64_t n, const uint32_t* ids, uint32_t* out_pos,
+                        std::chrono::steady_clock::time_point t0) {
+    dpq::ScanProgram& P = ix->prog;
+    cudaStream_t st = ix->stream;
+    const int M = P.M, cs = P.cstride;
+    const int64_t n_old = P.n_local, n_new = n_old + n;
+    const uint32_t first = (uint32_t)(P.base_pos + n_old);
+    const bool table = ix->has_pos2id || ids;
+    int rc;
+    // scratch: [keys 2n][values 2n][ids n][tail ids n][positions n], then the sort's
+    size_t tmp_bytes = 0;
+    if (ix->opt_add_order) CU(dpq::sort_add_batch(nullptr, n, M, cs, nullptr, nullptr, nullptr, &tmp_bytes, st));
+    const size_t n4 = ((size_t)n * 4 + 15) / 16 * 16;
+    const size_t off_vals = (size_t)n * 16, off_ids = off_vals + 2 * n4, off_tail = off_ids + n4, off_pos = off_tail + n4,
+                 off_tmp = off_pos + n4;
+    Scratch s;
+    if ((rc = s.b.ensure(off_tmp + tmp_bytes + 16))) return rc;
+    char* base = s.b.as<char>();
+    uint32_t* d_ids = ids ? reinterpret_cast<uint32_t*>(base + off_ids) : nullptr;
+    uint32_t* d_tail = table ? reinterpret_cast<uint32_t*>(base + off_tail) : nullptr;
+    uint32_t* d_pos = reinterpret_cast<uint32_t*>(base + off_pos);
+    if (ids) CU(cudaMemcpyAsync(d_ids, ids, (size_t)n * 4, cudaMemcpyDefault, st));
+    const uint32_t* perm = nullptr;
+    if (ix->opt_add_order) {
+        uint32_t* vals = reinterpret_cast<uint32_t*>(base + off_vals);
+        CU(dpq::sort_add_batch(d_in, n, M, cs, s.b.as<uint64_t>(), vals, base + off_tmp, &tmp_bytes, st));
+        perm = vals + n;
+    }
+    // room for the new nodes (and a zero pad word: the latency scan reads nodes in pairs)
+    if ((rc = grow(ix->d_codes, (size_t)n_old * cs, (size_t)(n_new + 1) * cs, st))) return rc;
+    CU(dpq::launch_add_gather(d_in, n, M, cs, perm, d_ids, first, ix->d_codes.as<uint8_t>() + (size_t)n_old * cs, d_tail, d_pos, st));
+    if (ix->d_dead.p && (rc = grow(ix->d_dead, (size_t)(n_old + 31) / 32 * 4, (size_t)(n_new + 31) / 32 * 4, st))) return rc;
+    if (table && ix->d_pos2id.p) {  // the device copy of the id table, once a search or a delete has uploaded it
+        if ((rc = grow(ix->d_pos2id, (size_t)n_old * 4, (size_t)n_new * 4, st))) return rc;
+        CU(cudaMemcpyAsync(ix->d_pos2id.as<uint32_t>() + n_old, d_tail, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+    }
+    std::vector<uint32_t> tail(table ? (size_t)n : 0);
+    if (table) CU(cudaMemcpyAsync(tail.data(), d_tail, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+    if (out_pos) CU(cudaMemcpyAsync(out_pos, d_pos, (size_t)n * 4, cudaMemcpyDefault, st));
+    CU(cudaStreamSynchronize(st));
+    if (table) {
+        if (!ix->has_pos2id) {  // the first add that names ids: the nodes so far keep id = position
+            ix->pos2id_host.resize((size_t)n_old);
+            for (int64_t i = 0; i < n_old; ++i) ix->pos2id_host[(size_t)i] = (uint32_t)(P.base_pos + i);
+            ix->has_pos2id = true;
+        }
+        ix->pos2id_host.insert(ix->pos2id_host.end(), tail.begin(), tail.end());
+    }
+    P.n_local = n_new;
+    ix->n_chunks = (int)((n_new + P.v2_chunk_nodes - 1) / P.v2_chunk_nodes);
+    ix->ops_bytes = (size_t)n_new * cs;
+    // the presample's gathered nodes were strided by the old n_local; presample_kernel tests dead bits at the new stride
+    ix->ps_R = 0;
+    ix->n_added += n;
+    ix->last_add_us = (int64_t)std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t0).count();
+    return DPQ_OK;
+}
+
+int dpq_index_add(dpq_index* ix, const uint8_t* codes, int64_t n, const uint32_t* ids, uint32_t* out_pos) {
+    const auto t0 = std::chrono::steady_clock::now();
+    bool done = true;
+    int rc = add_check(ix, codes, n, "dpq_index_add", &done);
+    if (rc || done) return rc;
+    CU(cudaSetDevice(ix->device));
+    const int M = ix->prog.M, K = ix->prog.K;
+    const uint8_t* d_in = codes;
+    Scratch staged;
+    if (!on_device(codes, ix->device)) {  // host memory, or another device's
+        if ((rc = staged.b.ensure((size_t)n * M))) return rc;
+        CU(cudaMemcpyAsync(staged.b.p, codes, (size_t)n * M, cudaMemcpyDefault, ix->stream));
+        d_in = staged.b.as<uint8_t>();
+    }
+    if (K < 256) {  // a code byte >= K would index past the tables; the check runs on the legacy stream
+        CU(cudaStreamSynchronize(ix->stream));
+        if ((rc = dpq::check_code_range(d_in, n, M, K))) return rc;
+    }
+    return append_nodes(ix, d_in, n, ids, out_pos, t0);
+}
+
+// Encoded on the device with the index's codebook by the kernels and path choice of dpq_encode (tensor cores for
+// Ds in {4, 8, 16} unless DPQ_ENCODE_TC=0), so the codes are bit-identical to its; input that is not on the
+// index's device is staged in chunks of at most 2^20 rows.
+int dpq_index_add_vectors(dpq_index* ix, const float* x, int64_t n, int D, const uint32_t* ids, uint32_t* out_pos) {
+    const auto t0 = std::chrono::steady_clock::now();
+    bool done = true;
+    int rc = add_check(ix, x, n, "dpq_index_add_vectors", &done);
+    if (rc || done) return rc;
+    const int M = ix->prog.M, K = ix->prog.K, Ds = ix->Ds;
+    if (!ix->d_cw.p || Ds < 1) return fail(DPQ_ERR_ARG, "dpq_index_add_vectors: no codebook (dpq_index_set_codebook first)");
+    if (D < 1 || D > M * Ds) return fail(DPQ_ERR_ARG, "dpq_index_add_vectors: D must be in 1 .. M * Ds");
+    CU(cudaSetDevice(ix->device));
+    cudaStream_t st = ix->stream;
+    const char* env = getenv("DPQ_ENCODE_TC");
+    const bool tc = dpq::encode_tc_supported(M, K, Ds) && !(env && env[0] == '0');
+    const bool on_dev = on_device(x, ix->device);  // else host memory or another device's: staged in chunks
+    const int64_t chunk = on_dev ? n : std::min<int64_t>(n, (int64_t)1 << 20);
+    Scratch s_codes, s_x, s_tc;
+    DevBuf &d_codes = s_codes.b, &d_x = s_x.b, &d_tc = s_tc.b;
+    if ((rc = d_codes.ensure((size_t)n * M)) || (!on_dev && (rc = d_x.ensure((size_t)chunk * D * 4)))) return rc;
+    int n_sms = 148;
+    if (tc) {  // [operand blocks][error word]
+        CU(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, ix->device));
+        if ((rc = d_tc.ensure(dpq::encode_tc_scratch_bytes(M) + 16))) return rc;
+        CU(cudaMemsetAsync(d_tc.as<char>() + dpq::encode_tc_scratch_bytes(M), 0, 4, st));
+    }
+    uint32_t* d_err = reinterpret_cast<uint32_t*>(d_tc.as<char>() + (tc ? dpq::encode_tc_scratch_bytes(M) : 0));
+    for (int64_t s0 = 0; s0 < n; s0 += chunk) {
+        const int64_t c = std::min(chunk, n - s0);
+        const float* src = x + (size_t)s0 * D;
+        if (!on_dev) {
+            CU(cudaMemcpyAsync(d_x.p, src, (size_t)c * D * 4, cudaMemcpyDefault, st));
+            src = d_x.as<float>();
+        }
+        uint8_t* dst = d_codes.as<uint8_t>() + (size_t)s0 * M;
+        if (tc) CU(dpq::launch_encode_tc(ix->d_cw.as<float>(), M, K, Ds, src, c, D, dst, d_tc.as<unsigned char>(), d_err, n_sms, st));
+        else CU(dpq::launch_encode(ix->d_cw.as<float>(), M, K, Ds, src, c, D, dst, st));
+        if (!on_dev) CU(cudaStreamSynchronize(st));  // the staging buffer is reused by the next chunk
+    }
+    if (tc) {
+        uint32_t err = 0;
+        CU(cudaMemcpyAsync(&err, d_err, 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (err) return fail(DPQ_ERR_CUDA, "dpq_index_add_vectors: a tensor-core completion barrier never fired");
+    }
+    return append_nodes(ix, d_codes.as<uint8_t>(), n, ids, out_pos, t0);
+}
 
 // slices of a pass over n_chunks chunks for n_groups query groups: whole waves of 148 one-CTA SMs and
 // whole rounds (warps x strands chunks) per item, as nearly as possible
@@ -1385,6 +1591,8 @@ int64_t dpq_index_stat(dpq_index* ix, const char* name) {
     if (n == "last_fallback") return ix->last_fallback;
     if (n == "n_deleted") return ix->n_deleted;
     if (n == "last_delete_us") return ix->last_delete_us;
+    if (n == "n_added") return ix->n_added;
+    if (n == "last_add_us") return ix->last_add_us;
     if (n.rfind("depth_hist_", 0) == 0) {
         size_t d = (size_t)atoi(n.c_str() + 11);
         return d < P.depth_hist.size() ? P.depth_hist[d] : 0;

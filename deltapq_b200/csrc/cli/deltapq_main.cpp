@@ -156,6 +156,19 @@ static int query(const Args& a, const std::string& dataset, const std::string& e
         DPQ_TRY(dpq_index_open_file(f_tree.c_str(), nodes_arg, M, K, 0, 1, &ix));
         DPQ_TRY(dpq_index_set_codebook(ix, cb.cw.data(), cb.Ds));
     }
+    const std::string added = a.str("-add", "");
+    if (!added.empty()) {  // extension: vectors (-ext format) appended to the open index with ids N + i
+        VecFile af;
+        if (!af.open(added, ext)) return die("cannot open " + added);
+        std::vector<float> xa;
+        const long long na = af.read(0x7FFFFFFFLL, xa);
+        if (af.D > Dp) return die("-add: vector dimension exceeds M*Ds of the codebook");
+        if (N < 0 || N + na > 0xFFFFFFFFLL) return die("-add needs -N, and ids N + i below 2^32 - 1");
+        std::vector<uint32_t> aid((size_t)na);
+        for (long long i = 0; i < na; ++i) aid[(size_t)i] = (uint32_t)(N + i);
+        if (mx) DPQ_TRY(dpq_multi_add_vectors(mx, xa.data(), na, af.D, aid.data(), nullptr));
+        else DPQ_TRY(dpq_index_add_vectors(ix, xa.data(), na, af.D, aid.data(), nullptr));
+    }
     const std::string deleted = a.str("-deleted", "");
     if (!deleted.empty()) {  // extension: vector ids (decimal, whitespace separated) that no query may return
         std::ifstream dfs(deleted);
@@ -201,7 +214,7 @@ int main(int argc, char** argv) {
     Args a{argc, argv};
     std::string dataset = a.str("-dataset", ""), ext = a.str("-ext", "fvecs"), task = a.str("-task", "approx_tree");
     int M = (int)a.num("-m", 8), K = (int)a.num("-k", 256);
-    if (dataset.empty()) return die("usage: deltapq -dataset DIR -task approx_tree|query|query_im|batch_query -m M -k K -h 1 -diff M -N N [-query_size Q] [-topk k] [-method 1|2] [-debug] [-results FILE] [-gpus N] [-parts P] [-repeat R] [-deleted FILE]");
+    if (dataset.empty()) return die("usage: deltapq -dataset DIR -task approx_tree|query|query_im|batch_query -m M -k K -h 1 -diff M -N N [-query_size Q] [-topk k] [-method 1|2] [-debug] [-results FILE] [-gpus N] [-parts P] [-repeat R] [-add FILE] [-deleted FILE]");
     if (task == "approx_tree") return approx_tree(a, dataset, M, K);
     if (task == "query" || task == "query_im" || task == "batch_query") return query(a, dataset, ext, M, K);
     return die("deltapq: task '" + task + "' is outside the B200 hot-path scope (approx_tree, query, query_im, batch_query)");

@@ -478,4 +478,19 @@ void launch_mark_dead(const uint32_t* d_ids, int64_t n_ids, const uint32_t* d_po
 // CUB radix sort of n ids (d_temp = null: *temp_bytes receives the scratch size and nothing runs)
 cudaError_t sort_ids(const uint32_t* d_in, uint32_t* d_out, int n, void* d_temp, size_t* temp_bytes, cudaStream_t st);
 
+// ---- appended nodes (add.cu): the layout of an add batch --------------------------------------------
+// Sorts the rows of d_codes [n][M] by their padded code word of nf bytes (subspace 0 most significant; ties by
+// input row, the sorts being stable).  d_keys: [2n], d_vals: [2n]; the order (input row of each appended node)
+// is left in d_vals + n.  d_temp = null: *temp_bytes receives the scratch size and nothing runs.
+cudaError_t sort_add_batch(const uint8_t* d_codes, int64_t n, int M, int nf, uint64_t* d_keys, uint32_t* d_vals, void* d_temp,
+                           size_t* temp_bytes, cudaStream_t st);
+// Appended node i = input row d_perm[i] (row i when d_perm is null): its code word padded to nf bytes goes to
+// d_out_codes [n][nf], its id (d_ids[row], or its position when d_ids is null) to d_out_ids [n] (skipped when
+// null), and its position first_pos + i to d_out_pos[row].
+cudaError_t launch_add_gather(const uint8_t* d_codes, int64_t n, int M, int nf, const uint32_t* d_perm, const uint32_t* d_ids,
+                              uint32_t first_pos, uint8_t* d_out_codes, uint32_t* d_out_ids, uint32_t* d_out_pos, cudaStream_t st);
+// secondary.cu: the SIMT encoder (any Ds)
+cudaError_t launch_encode(const float* d_cw, int M, int K, int Ds, const float* d_x, int64_t n, int D, uint8_t* d_codes,
+                          cudaStream_t st);
+
 }  // namespace dpq

@@ -79,6 +79,7 @@ struct dpq_multi {
     void* h_stage = nullptr;
     size_t h_cap = 0;
     std::vector<uint32_t> pos2id;  // position -> vector id over the whole position space
+    size_t last = 0;               // the index whose positions end the position space: it takes every add
     int64_t open_us = 0, nccl_us = 0;  // wall time of opening the shards / of ncclCommInitAll
 };
 
@@ -206,6 +207,7 @@ int dpq_multi_open_file(const char* tree_path, const char* qnode_path, int M, in
             if (rcs[(size_t)r]) rc = dpq::api_fail(rcs[(size_t)r], errs[(size_t)r]);
     }
     m->open_us = std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t_open0).count();
+    m->last = (size_t)n_gpus - 1;
     if (!rc) rc = finish_multi_open(m);
     if (!rc && qnode_path) {
         const int64_t n_codes = dpq_index_stat(m->ix[0], "n_codes");
@@ -258,6 +260,8 @@ int dpq_multi_open_parts(const char* const* tree_paths, const char* const* qnode
             if (rcs[(size_t)p]) rc = dpq::api_fail(rcs[(size_t)p], errs[(size_t)p]);
         for (int p = 0; p < n_parts && !rc; ++p)
             span = std::max<int64_t>(span, first_pos[p] + dpq_index_stat(m->ix[(size_t)p], "n_codes"));
+        for (int p = 0; p < n_parts; ++p)
+            if (first_pos[p] >= first_pos[m->last]) m->last = (size_t)p;
     }
     if (!rc) rc = finish_multi_open(m);
     if (!rc && qnode_paths) {  // ids of part p = first_pos[p] + its own vec_id (parts are id ranges)
@@ -418,6 +422,47 @@ static int multi_mark_dead(dpq_multi* m, const uint32_t* ids, int64_t n, bool se
 int dpq_multi_delete(dpq_multi* m, const uint32_t* ids, int64_t n) { return multi_mark_dead(m, ids, n, true, "dpq_multi_delete"); }
 int dpq_multi_undelete(dpq_multi* m, const uint32_t* ids, int64_t n) {
     return multi_mark_dead(m, ids, n, false, "dpq_multi_undelete");
+}
+
+// The index that ends the position space takes the batch with ids = its positions (shard and part indexes have no
+// id table); the handle's own table maps those positions to the caller's ids.
+// D = 0: data are codes; else vectors of D floats.
+static int multi_add(dpq_multi* m, const void* data, int64_t n, int D, const uint32_t* ids, uint32_t* out_pos, const char* what) {
+    int rc = dpq::api_check_device();
+    if (rc) return rc;
+    if (!m) return dpq::api_fail(DPQ_ERR_ARG, std::string(what) + ": null handle");
+    if (n < 0 || (n > 0 && !data)) return dpq::api_fail(DPQ_ERR_ARG, std::string(what) + ": input is null or n < 0");
+    if (n > 0x7FFFFFFFLL) return dpq::api_fail(DPQ_ERR_ARG, std::string(what) + ": more than 2^31 - 1 rows in one call");
+    if (D < 0) return dpq::api_fail(DPQ_ERR_ARG, std::string(what) + ": D must be >= 1");
+    if (n == 0) return DPQ_OK;
+    dpq_index* ix = m->ix[m->last];
+    std::vector<uint32_t> pos((size_t)n), hid;
+    if (ids) {  // host or device pointer
+        hid.resize((size_t)n);
+        CUM(cudaMemcpy(hid.data(), ids, (size_t)n * 4, cudaMemcpyDefault));
+    }
+    CUM(cudaSetDevice(m->dev[m->last]));
+    rc = D ? dpq_index_add_vectors(ix, static_cast<const float*>(data), n, D, nullptr, pos.data())
+           : dpq_index_add(ix, static_cast<const uint8_t*>(data), n, nullptr, pos.data());
+    if (rc) return rc;
+    if (ids || !m->pos2id.empty()) {
+        const size_t end = (size_t)*std::max_element(pos.begin(), pos.end()) + 1, old = m->pos2id.size();
+        if (end > old) {
+            m->pos2id.resize(end);
+            for (size_t p = old; p < end; ++p) m->pos2id[p] = (uint32_t)p;
+        }
+        for (size_t j = 0; j < pos.size(); ++j) m->pos2id[pos[j]] = ids ? hid[j] : pos[j];
+    }
+    if (out_pos) CUM(cudaMemcpy(out_pos, pos.data(), (size_t)n * 4, cudaMemcpyDefault));
+    CUM(cudaSetDevice(0));
+    return DPQ_OK;
+}
+
+int dpq_multi_add(dpq_multi* m, const uint8_t* codes, int64_t n, const uint32_t* ids, uint32_t* out_pos) {
+    return multi_add(m, codes, n, 0, ids, out_pos, "dpq_multi_add");
+}
+int dpq_multi_add_vectors(dpq_multi* m, const float* x, int64_t n, int D, const uint32_t* ids, uint32_t* out_pos) {
+    return multi_add(m, x, n, D < 1 ? -1 : D, ids, out_pos, "dpq_multi_add_vectors");
 }
 
 int64_t dpq_multi_stat(dpq_multi* m, int rank, const char* name) {

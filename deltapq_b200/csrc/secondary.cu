@@ -113,6 +113,10 @@ __global__ void u8_to_float_kernel(const uint8_t* __restrict__ src, int64_t n, i
     dst[i] = (float)src[v * stride + skip + (i - v * D)];
 }
 
+}  // namespace
+
+namespace dpq {  // also used by dpq_index_add_vectors (api.cu)
+
 cudaError_t launch_encode(const float* d_cw, int M, int K, int Ds, const float* d_x, int64_t n, int D,
                           uint8_t* d_codes, cudaStream_t st) {
     dim3 grid((unsigned)((n + 255) / 256), (unsigned)M), block(256);
@@ -138,6 +142,10 @@ cudaError_t launch_encode(const float* d_cw, int M, int K, int Ds, const float* 
 #undef DPQ_ENC
     return cudaGetLastError();
 }
+
+}  // namespace dpq
+
+namespace {
 
 // ------------------------------------------------------------------------ edge diffs ---
 __global__ void edge_diff_kernel(const uint8_t* __restrict__ codes, int M, const uint32_t* __restrict__ edges,
@@ -438,7 +446,7 @@ struct Encoder {
             CU(dpq::launch_encode_tc((const float*)d_cw.p, M, K, Ds, d_x, n, D, d_codes, (unsigned char*)d_scratch.p,
                                      (uint32_t*)d_err.p, n_sms, 0));
         else
-            CU(launch_encode((const float*)d_cw.p, M, K, Ds, d_x, n, D, d_codes, 0));
+            CU(dpq::launch_encode((const float*)d_cw.p, M, K, Ds, d_x, n, D, d_codes, 0));
         CU(cudaEventRecord(ev[1], 0));
         CU(cudaEventSynchronize(ev[1]));
         float t = 0.0f;

@@ -99,7 +99,8 @@ int dpq_index_set_stream(dpq_index* idx, void* cuda_stream);
  * "refine" (stride of a second, denser sample pass; automatic on shards above 16.8M nodes), "stight"
  * (percent of the presample cap the first sampled pass accepts, default 100), "presample", "parts8",
  * "levels8", "bcap8", "warps8", "coarse_min" (coarse search); "latency" (-1 auto, 0 off, 1 on: lanes =
- * nodes scan for a handful of queries);
+ * nodes scan for a handful of queries); "add_order" (1 default: an add batch is laid out sorted by code word, 0:
+ * in input order);
  * first-generation engine only: "pack" (1 = 31-bit, 2 = 2x15-bit filter). */
 int dpq_index_set_option(dpq_index* idx, const char* name, int64_t value);
 
@@ -118,6 +119,30 @@ int dpq_index_set_option(dpq_index* idx, const char* name, int64_t value);
  * shard currently deleted; "last_delete_us": host wall time of the last call. */
 int dpq_index_delete(dpq_index* idx, const uint32_t* ids, int64_t n);
 int dpq_index_undelete(dpq_index* idx, const uint32_t* ids, int64_t n);
+
+/* Adds vectors to an open index (an extension, like deletion).  codes is [n][M]; x is [n][D] floats with
+ * D <= M*Ds, zero-padded like dpq_encode and encoded on the device with this index's codebook
+ * (dpq_index_set_codebook first, else DPQ_ERR_ARG) by the same kernels, so the codes are bit-identical to
+ * dpq_encode's.  codes / x / ids / out_pos may be host pointers or device pointers of any device: input that is
+ * not on the index's device is copied there first (no peer access is needed).  ids may be NULL: a node's id is then
+ * its position.  out_pos (may be NULL) receives the position given to input row i at out_pos[i].
+ * Positions: appended nodes continue this index's range, base_pos + n_local, + 1, ... and every search path
+ * scores them exactly like tree nodes.  Only an index whose range ends the position space accepts adds: a whole
+ * tree, the last shard (rank = n_ranks - 1, also when it is empty) or a forest part; another shard returns
+ * DPQ_ERR_ARG.  A lone forest part continues at first_pos + n_codes + j: keeping those positions clear of the next
+ * part is the caller's job (dpq_multi_add does it).  A position reaching 0xFFFFFFFF is DPQ_ERR_ARG and changes
+ * nothing; so are n > 2^31 - 1, a null codes / x with n > 0, a code byte >= K and the first-generation engine
+ * (DPQ_ENGINE=1).  n = 0 does nothing.
+ * Layout: each call's batch is sorted on the device by code word (subspace 0 most significant, ties by input
+ * row) and appended in that order, so that neighbouring positions share centroids as DFS neighbours of the tree
+ * do; set_option("add_order", 0) appends in input order instead.
+ * Ids: an index without a pos2id table keeps none while ids is NULL (id = position); the first add that names
+ * ids creates one, identity over the nodes it already had.  Duplicate ids are allowed: dpq_index_delete removes
+ * every node that carries the id, and a node added after its id was deleted is live (the bitmap is per node).
+ * The call runs on the index's stream and returns once the change is complete.  Adds are not written to any
+ * file.  Stats: "n_added" (appended nodes), "last_add_us"; "n_local" counts appended nodes, "n_codes" does not. */
+int dpq_index_add(dpq_index* idx, const uint8_t* codes, int64_t n, const uint32_t* ids, uint32_t* out_pos);
+int dpq_index_add_vectors(dpq_index* idx, const float* x, int64_t n, int D, const uint32_t* ids, uint32_t* out_pos);
 
 /* Replaces the per-query loop dmain:328-344 calling
  * query_processing_scan_compressed_codes_opt_o_direct (DCAT.h:2805) /
@@ -167,6 +192,13 @@ int64_t dpq_multi_stat(dpq_multi* m, int rank, const char* name); /* dpq_index_s
  * part is given the same list and keeps the nodes it holds. */
 int dpq_multi_delete(dpq_multi* m, const uint32_t* ids, int64_t n);
 int dpq_multi_undelete(dpq_multi* m, const uint32_t* ids, int64_t n);
+/* dpq_index_add / _add_vectors for the handle: the whole batch goes to the index that ends the position space
+ * (the last shard, or the part with the largest first_pos) and the new positions continue the global space.
+ * The handle's id table grows with them (created as identity when it was empty and ids are given), so that
+ * dpq_multi_search reports the ids and dpq_multi_delete takes them.  As for dpq_index_add, the inputs may be on
+ * any device.  Every add lands on that one GPU: a known imbalance of the search load. */
+int dpq_multi_add(dpq_multi* m, const uint8_t* codes, int64_t n, const uint32_t* ids, uint32_t* out_pos);
+int dpq_multi_add_vectors(dpq_multi* m, const float* x, int64_t n, int D, const uint32_t* ids, uint32_t* out_pos);
 void dpq_multi_close(dpq_multi* m);
 
 /* Raw device allocation helpers for hosts without a CUDA binding (ctypes, cgo, JNI). */
@@ -186,7 +218,7 @@ int dpq_free_host(void* hptr);
  * "last_coarse" (1 when the last search used the sample -> 8-bit coarse scan -> exact re-score
  * path), "last_latency" (1: latency mode), "last_scan8_us" / "sum_scan8_ns" (the coarse scan kernel
  * alone; in latency mode the full scan1 pass), "device_bytes_per_node", "engine"; "n_deleted",
- * "last_delete_us" (dpq_index_delete). */
+ * "last_delete_us" (dpq_index_delete); "n_added", "last_add_us" (dpq_index_add). */
 int64_t dpq_index_stat(dpq_index* idx, const char* name);
 
 void dpq_index_close(dpq_index* idx);
