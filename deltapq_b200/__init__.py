@@ -28,6 +28,7 @@ SYMBOLS = [
     "dpq_tree_free", "dpq_multi_open_file", "dpq_multi_set_codebook", "dpq_multi_search", "dpq_multi_stat",
     "dpq_multi_close", "dpq_index_delete", "dpq_index_undelete", "dpq_multi_delete", "dpq_multi_undelete",
     "dpq_index_add", "dpq_index_add_vectors", "dpq_multi_add", "dpq_multi_add_vectors",
+    "dpq_index_compact", "dpq_multi_compact",
 ]
 
 
@@ -115,6 +116,8 @@ def lib():
         getattr(L, name).argtypes = [vp, vp, i64, vp, vp]
     for name in ("dpq_index_add_vectors", "dpq_multi_add_vectors"):
         getattr(L, name).argtypes = [vp, vp, i64, i32, vp, vp]
+    L.dpq_index_compact.argtypes = [vp, C.POINTER(vp)]
+    L.dpq_multi_compact.argtypes = [vp]
     _lib = L
     return L
 
@@ -289,6 +292,17 @@ class DeltaTreeIndex:
         """dpq_index_add_vectors: x [n][D] encoded with the index's codebook and appended; returns the positions."""
         return _add(lib().dpq_index_add_vectors, self._h, x, ids, D=np.asarray(x).shape[1])
 
+    def compact(self, want=("payload", "vec_id", "qnodes")):
+        """dpq_index_compact: the tree is rebuilt over the live nodes (positions renumbered, ids kept).  Returns the
+        new tree's arrays by name, as tree_build does (vec_id = the carried ids; "qnodes" at M = 8 only), or None
+        with want=None, in which case only the index's id table leaves the device."""
+        if want is None:
+            _check(lib().dpq_index_compact(self._h, None))
+            return None
+        t = C.c_void_p()
+        _check(lib().dpq_index_compact(self._h, C.byref(t)))
+        return _tree_out(t, self.M, want)
+
     def search_device(self, d_queries_ptr, Q, topk, d_out_ptr):
         _check(lib().dpq_index_search_device(self._h, d_queries_ptr, Q, topk, d_out_ptr))
 
@@ -349,6 +363,10 @@ class MultiIndex:
 
     def add_vectors(self, x, ids=None):
         return _add(lib().dpq_multi_add_vectors, self._h, x, ids, D=np.asarray(x).shape[1])
+
+    def compact(self):
+        """dpq_multi_compact: one tree over the live nodes, dealt to the GPUs again (forest: every part rebuilt)."""
+        _check(lib().dpq_multi_compact(self._h))
 
     def stat(self, rank, name):
         return int(lib().dpq_multi_stat(self._h, rank, name.encode()))

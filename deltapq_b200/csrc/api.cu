@@ -10,10 +10,12 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <vector>
 
 #include "../../include/dpq.h"
+#include "compact.cuh"
 #include "encode_tc.cuh"
 #include "kernels.cuh"
 #include "tree_internal.h"
@@ -150,6 +152,10 @@ struct dpq_index {
     int opt_add_order = 1;     // 1: an add batch is laid out sorted by code word; 0: in input order
     int64_t n_added = 0;
     int64_t last_add_us = 0;   // host wall clock of the last dpq_index_add / _add_vectors (ends in a stream sync)
+    int n_ranks = 1;           // shards the tree was split into when this index was opened
+    std::vector<float> cw_host;  // the codebook again: a compaction's layout builds its centroid tables on the host
+    // host wall clock of the last dpq_index_compact: whole call, gather, edge search, layout (each ends in a sync)
+    int64_t compact_us[4] = {0, 0, 0, 0};
 };
 
 namespace {
@@ -373,6 +379,7 @@ static int open_common(const uint8_t* payload, int64_t n_bytes, int64_t n_codes,
         return fail(DPQ_ERR_FORMAT, "dpq_index_open: " + err);
     }
     ix->ends_range = rank == n_ranks - 1;
+    ix->n_ranks = n_ranks;
     if (first_pos) {  // one tree of a forest: every position this index reports is shifted
         ix->pos_shift = first_pos;
         ix->prog.base_pos += first_pos;
@@ -528,21 +535,18 @@ int dpq_index_open_tree_shard(dpq_tree* t, int rank, int n_ranks, dpq_index** ou
     return open_tree_shard_impl(t, rank, n_ranks, 0, out);
 }
 
-// device-resident tree -> index of one shard; first_pos shifts every reported position (forest parts)
-static int open_tree_shard_impl(dpq_tree* t, int rank, int n_ranks, int64_t first_pos, dpq_index** out) {
+// Fills ix (device, stream set; nothing loaded yet) with shard `rank` of `n_ranks` of a device-resident tree;
+// first_pos shifts every reported position (forest parts).  On failure the caller closes ix.
+static int load_tree_shard(dpq_index* ix, dpq_tree* t, int rank, int n_ranks, int64_t first_pos) {
     const int M = t->M, K = t->K;
     const int64_t n = t->n;
-    if (first_pos < 0 || first_pos + n > 0xFFFFFFFFLL) return fail(DPQ_ERR_ARG, "dpq_index_open: positions must stay below 2^32 - 1");
-    int rc = check_device();
-    if (rc) return rc;
-    if (g_device != t->device) return fail(DPQ_ERR_ARG, "dpq_index_open_tree_shard: the tree lives on another device");
+    int rc;
     std::vector<int64_t> bounds, bytes;
     if ((rc = dpq::tree_shard_bounds(t, n_ranks, &bounds, &bytes))) return rc;
     int64_t lo = bounds[(size_t)rank], hi = bounds[(size_t)rank + 1];
     if (hi == lo) lo = hi = n;  // an empty shard reports base_pos = n_codes like the stream reader (program.cpp)
-    dpq_index* ix = new dpq_index();
-    ix->device = g_device;
     ix->ends_range = rank == n_ranks - 1;
+    ix->n_ranks = n_ranks;
     dpq::ScanProgram& P = ix->prog;
     P.M = M;
     P.K = K;
@@ -562,16 +566,9 @@ static int open_tree_shard_impl(dpq_tree* t, int rank, int n_ranks, int64_t firs
         P.n_diffs = bytes[(size_t)rank] - (rank == 0 ? M : 0) - (int64_t)((M + 7) / 8) * recs - odd;
     }
     int64_t hist[17] = {0};
-    auto bail = [&](int code) {
-        dpq_index_close(ix);
-        return code;
-    };
-    if (cudaSetDevice(ix->device) != cudaSuccess ||
-        cudaStreamCreateWithFlags(&ix->stream, cudaStreamNonBlocking) != cudaSuccess)
-        return bail(fail(DPQ_ERR_CUDA, "dpq_index_open_tree_shard: stream setup failed"));
-    if ((rc = dpq::depth_hist_device(ix->device, (const uint8_t*)t->d_depth + lo, P.n_local, hist))) return bail(rc);
+    if ((rc = dpq::depth_hist_device(ix->device, (const uint8_t*)t->d_depth + lo, P.n_local, hist))) return rc;
     P.depth_hist.assign(hist, hist + 17);
-    if ((rc = ix->d_codes.ensure((size_t)std::max<int64_t>(P.n_local, 1) * P.cstride))) return bail(rc);
+    if ((rc = ix->d_codes.ensure((size_t)std::max<int64_t>(P.n_local, 1) * P.cstride))) return rc;
     cudaError_t e = cudaSuccess;
     const uint8_t* src = (const uint8_t*)t->d_codes_by_pos + (size_t)lo * M;
     if (P.n_local > 0) {
@@ -580,7 +577,7 @@ static int open_tree_shard_impl(dpq_tree* t, int rank, int n_ranks, int64_t firs
         else
             e = dpq::launch_pad_codes(src, P.n_local, M, P.cstride, ix->d_codes.as<uint8_t>(), ix->stream);
     }
-    if ((rc = ix->d_ops.ensure(16)) || (rc = ix->d_chunks.ensure(16)) || (rc = ix->d_anc.ensure(16))) return bail(rc);
+    if ((rc = ix->d_ops.ensure(16)) || (rc = ix->d_chunks.ensure(16)) || (rc = ix->d_anc.ensure(16))) return rc;
     if (t->d_vec_id) {
         ix->pos2id_host.resize((size_t)P.n_local);
         if (e == cudaSuccess && P.n_local > 0)
@@ -589,9 +586,29 @@ static int open_tree_shard_impl(dpq_tree* t, int rank, int n_ranks, int64_t firs
         ix->has_pos2id = true;
     }
     if (e == cudaSuccess) e = cudaStreamSynchronize(ix->stream);
-    if (e != cudaSuccess) return bail(fail(DPQ_ERR_CUDA, std::string("dpq_index_open_tree_shard: ") + cudaGetErrorString(e)));
+    if (e != cudaSuccess) return fail(DPQ_ERR_CUDA, std::string("dpq_index_open_tree_shard: ") + cudaGetErrorString(e));
     ix->n_chunks = (int)((P.n_local + P.v2_chunk_nodes - 1) / P.v2_chunk_nodes);
     ix->ops_bytes = (size_t)P.n_local * P.cstride;
+    return DPQ_OK;
+}
+
+// device-resident tree -> index of one shard; first_pos shifts every reported position (forest parts)
+static int open_tree_shard_impl(dpq_tree* t, int rank, int n_ranks, int64_t first_pos, dpq_index** out) {
+    if (first_pos < 0 || first_pos + t->n > 0xFFFFFFFFLL) return fail(DPQ_ERR_ARG, "dpq_index_open: positions must stay below 2^32 - 1");
+    int rc = check_device();
+    if (rc) return rc;
+    if (g_device != t->device) return fail(DPQ_ERR_ARG, "dpq_index_open_tree_shard: the tree lives on another device");
+    dpq_index* ix = new dpq_index();
+    ix->device = g_device;
+    if (cudaSetDevice(ix->device) != cudaSuccess ||
+        cudaStreamCreateWithFlags(&ix->stream, cudaStreamNonBlocking) != cudaSuccess) {
+        dpq_index_close(ix);
+        return fail(DPQ_ERR_CUDA, "dpq_index_open_tree_shard: stream setup failed");
+    }
+    if ((rc = load_tree_shard(ix, t, rank, n_ranks, first_pos))) {
+        dpq_index_close(ix);
+        return rc;
+    }
     *out = ix;
     return DPQ_OK;
 }
@@ -610,9 +627,11 @@ int dpq_index_set_codebook(dpq_index* ix, const float* cw, int Ds) {
     if (!ix || !cw || Ds < 1) return fail(DPQ_ERR_ARG, "dpq_index_set_codebook: bad argument");
     CU(cudaSetDevice(ix->device));
     ix->Ds = Ds;
-    int rc = upload(ix->d_cw, cw, (size_t)ix->prog.M * ix->prog.K * Ds * sizeof(float), ix->stream);
+    const size_t n = (size_t)ix->prog.M * ix->prog.K * Ds;
+    int rc = upload(ix->d_cw, cw, n * sizeof(float), ix->stream);
     if (rc) return rc;
     CU(cudaStreamSynchronize(ix->stream));
+    ix->cw_host.assign(cw, cw + n);
     return DPQ_OK;
 }
 
@@ -660,6 +679,16 @@ int dpq_index_set_option(dpq_index* ix, const char* name, int64_t v) {
     return DPQ_OK;
 }
 
+// The device copy of the id table, uploaded on the index's stream the first time a search, a delete or a compaction
+// needs it; later changes (dpq_index_add) keep both copies in step.
+static int upload_pos2id(dpq_index* ix) {
+    if (!ix->has_pos2id || ix->d_pos2id.p) return DPQ_OK;
+    int rc = ix->d_pos2id.ensure(std::max<size_t>(ix->pos2id_host.size(), 1) * 4);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(ix->d_pos2id.p, ix->pos2id_host.data(), ix->pos2id_host.size() * 4, cudaMemcpyHostToDevice, ix->stream));
+    return DPQ_OK;
+}
+
 // dpq_index_delete / dpq_index_undelete: the ids are sorted on the device, then every 32-position word of the
 // bitmap is rebuilt from a binary search of its nodes' ids (dead.cu).  The caller's stream orders the change
 // before every later search; the call returns once it is complete.
@@ -685,10 +714,7 @@ static int mark_dead(dpq_index* ix, const uint32_t* ids, int64_t n, bool set, co
         if ((rc = ix->d_dead.ensure(std::max<size_t>(words, 1) * 4))) return rc;
         CU(cudaMemsetAsync(ix->d_dead.p, 0, ix->d_dead.cap, st));
     }
-    if (ix->has_pos2id && !ix->d_pos2id.p) {  // the same id table the host-buffer search uploads
-        if ((rc = ix->d_pos2id.ensure(std::max<size_t>(ix->pos2id_host.size(), 1) * 4))) return rc;
-        CU(cudaMemcpyAsync(ix->d_pos2id.p, ix->pos2id_host.data(), ix->pos2id_host.size() * 4, cudaMemcpyHostToDevice, st));
-    }
+    if ((rc = upload_pos2id(ix))) return rc;
     // [n raw ids][n sorted ids][count], then the sort's scratch
     const size_t ids_bytes = ((size_t)n * 4 + 15) / 16 * 16;
     size_t tmp_bytes = 0;
@@ -869,6 +895,141 @@ int dpq_index_add_vectors(dpq_index* ix, const float* x, int64_t n, int D, const
         if (err) return fail(DPQ_ERR_CUDA, "dpq_index_add_vectors: a tensor-core completion barrier never fired");
     }
     return append_nodes(ix, d_codes.as<uint8_t>(), n, ids, out_pos, t0);
+}
+
+// The live nodes of ix in ascending local position, gathered on its stream (compact.cu): *d_codes [n_live][M]
+// unpadded, *d_ids [n_live] the id each node reports (pos2id[pos], else its position).  Both are cudaMalloc'ed for
+// the caller to free; with no live node both stay null.  Returns once the device work is complete.
+static int live_nodes(dpq_index* ix, uint8_t** d_codes, uint32_t** d_ids, int64_t* n_live) {
+    *d_codes = nullptr;
+    *d_ids = nullptr;
+    *n_live = 0;
+    const dpq::ScanProgram& P = ix->prog;
+    cudaStream_t st = ix->stream;
+    const int64_t n = P.n_local, words = (n + 31) / 32;
+    int rc;
+    if ((rc = upload_pos2id(ix))) return rc;
+    const uint32_t* dead = ix->dead();
+    Scratch off, codes, ids;  // off: [live offsets words + 1][live counts words + 1][the scan's scratch]
+    int64_t count = n;
+    if (dead) {
+        size_t tmp = 0;
+        CU(dpq::count_live(dead, n, nullptr, nullptr, nullptr, &tmp, st));
+        const size_t off_bytes = ((size_t)(words + 1) * 4 + 255) / 256 * 256;
+        if ((rc = off.b.ensure(2 * off_bytes + tmp))) return rc;
+        CU(dpq::count_live(dead, n, reinterpret_cast<uint32_t*>(off.b.as<char>() + off_bytes), off.b.as<uint32_t>(),
+                           off.b.as<char>() + 2 * off_bytes, &tmp, st));
+        uint32_t c = 0;
+        CU(cudaMemcpyAsync(&c, off.b.as<uint32_t>() + words, 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        count = c;
+    }
+    if (count == 0) return DPQ_OK;
+    if ((rc = codes.b.ensure((size_t)count * P.M)) || (rc = ids.b.ensure((size_t)count * 4))) return rc;
+    CU(dpq::gather_live(ix->d_codes.as<uint8_t>(), P.cstride, n, P.M, dead, off.b.as<uint32_t>(),
+                        ix->has_pos2id ? ix->d_pos2id.as<uint32_t>() : nullptr, (uint32_t)P.base_pos, codes.b.as<uint8_t>(),
+                        ids.b.as<uint32_t>(), st));
+    CU(cudaStreamSynchronize(st));
+    *d_codes = codes.b.as<uint8_t>();
+    *d_ids = ids.b.as<uint32_t>();
+    codes.b.p = ids.b.p = nullptr;  // handed to the caller
+    *n_live = count;
+    return DPQ_OK;
+}
+
+// Gather the live nodes, build their tree on the device (the edge search and layout of dpq_tree_build_device with
+// the defaults of `deltapq -task approx_tree`: -h 1, -method 1), map its vec_id to the carried ids, load it into a
+// new index state on the same stream, and only then swap that state in: a failure at any step leaves ix as it was.
+int dpq_index_compact(dpq_index* ix, dpq_tree** out_tree) {
+    using clk = std::chrono::steady_clock;
+    const auto t0 = clk::now();
+    auto us = [](clk::time_point a, clk::time_point b) { return (int64_t)std::chrono::duration_cast<std::chrono::microseconds>(b - a).count(); };
+    if (out_tree) *out_tree = nullptr;
+    int rc = check_device();
+    if (rc) return rc;
+    if (!ix) return fail(DPQ_ERR_ARG, "dpq_index_compact: null index");
+    const dpq::ScanProgram& P = ix->prog;
+    if (!P.v2)
+        return fail(DPQ_ERR_ARG,
+                    "dpq_index_compact: compaction needs the code-array engine (this index runs the first-generation engine, DPQ_ENGINE=1)");
+    if (ix->n_ranks > 1)
+        return fail(DPQ_ERR_ARG, "dpq_index_compact: this index is one shard of a tree split over several ranks (dpq_multi_compact compacts those)");
+    if (!ix->d_cw.p || ix->cw_host.empty()) return fail(DPQ_ERR_ARG, "dpq_index_compact: no codebook (dpq_index_set_codebook first)");
+    const int M = P.M, K = P.K;
+    CU(cudaSetDevice(ix->device));
+    struct Restore {  // the build runs on the thread's selected device, which is the index's for the call's duration
+        int d;
+        ~Restore() { g_device = d; }
+    } restore{g_device};
+    g_device = ix->device;
+    uint8_t* d_live = nullptr;
+    uint32_t* d_ids = nullptr;
+    int64_t n_live = 0;
+    rc = live_nodes(ix, &d_live, &d_ids, &n_live);
+    Scratch live_codes, live_ids;  // released on every return path
+    live_codes.b.p = d_live;
+    live_ids.b.p = d_ids;
+    if (rc) return rc;
+    if (n_live == 0) return fail(DPQ_ERR_ARG, "dpq_index_compact: every node is deleted (a tree needs at least one node)");
+    const auto t1 = clk::now();
+    std::unique_ptr<dpq_tree> t(new dpq_tree());
+    t->M = M;
+    t->K = K;
+    t->n = n_live;
+    uint32_t* d_edges = nullptr;
+    rc = dpq::find_edges_device(d_live, n_live, M, K, 1, 1, &d_edges, &t->root);
+    const auto t2 = clk::now();
+    if (!rc) rc = dpq::layout_tree_device(d_live, n_live, M, K, ix->cw_host.data(), ix->Ds, t.get(), d_edges, true, out_tree != nullptr);
+    if (d_edges) cudaFree(d_edges);
+    const auto t3 = clk::now();
+    if (rc) return rc;
+    t->edge_us = us(t1, t2);
+    t->layout_us = us(t2, t3);
+    // the layout ended in a device synchronisation; the new state is filled on the index's stream
+    CU(dpq::map_tree_ids(static_cast<uint32_t*>(t->d_vec_id), n_live, d_ids, ix->stream));
+    dpq_index* nx = new dpq_index();
+    nx->device = ix->device;
+    nx->stream = ix->stream;
+    nx->own_stream = false;
+    rc = load_tree_shard(nx, t.get(), 0, 1, ix->pos_shift);  // ends in a stream synchronisation
+    if (!rc && out_tree) {  // the host form dpq_tree_build returns (the QNode fields came with the layout)
+        t->vec_id.resize((size_t)n_live);
+        t->depth.resize((size_t)n_live);
+        t->codes_by_pos.resize((size_t)n_live * M);
+        t->payload.resize((size_t)t->payload_bytes);
+        if (!(rc = dpq::tree_copy_device(t.get(), t->d_vec_id, t->vec_id.data(), t->vec_id.size() * 4)) &&
+            !(rc = dpq::tree_copy_device(t.get(), t->d_depth, t->depth.data(), t->depth.size())) &&
+            !(rc = dpq::tree_copy_device(t.get(), t->d_codes_by_pos, t->codes_by_pos.data(), t->codes_by_pos.size())))
+            rc = dpq::tree_copy_device(t.get(), t->d_payload, t->payload.data(), t->payload.size());
+    }
+    if (rc) {
+        dpq_index_close(nx);
+        return rc;
+    }
+    // swap: positions renumbered from base_pos, ids carried, tombstones and the appended tail gone
+    std::swap(ix->d_codes, nx->d_codes);
+    ix->prog = nx->prog;
+    ix->pos2id_host.swap(nx->pos2id_host);
+    ix->has_pos2id = true;
+    ix->n_chunks = nx->n_chunks;
+    ix->ops_bytes = nx->ops_bytes;
+    ix->d_pos2id.release();  // uploaded again from pos2id_host when a search or a delete needs it
+    ix->d_dead.release();
+    ix->n_deleted = 0;
+    ix->n_added = 0;
+    ix->ps_R = 0;  // the presample's nodes were gathered from the old code array
+    dpq_index_close(nx);  // frees the old code array
+    if (out_tree) {
+        dpq::tree_release_device(t.get());
+        t->on_device = false;
+        *out_tree = t.release();
+    }
+    const auto t4 = clk::now();
+    ix->compact_us[0] = us(t0, t4);
+    ix->compact_us[1] = us(t0, t1);
+    ix->compact_us[2] = us(t1, t2);
+    ix->compact_us[3] = us(t2, t3);
+    return DPQ_OK;
 }
 
 // slices of a pass over n_chunks chunks for n_groups query groups: whole waves of 148 one-CTA SMs and
@@ -1484,10 +1645,7 @@ int dpq_index_search(dpq_index* ix, const float* queries, int Q, int topk, uint3
     uint32_t* const o_dist = mapped(out_dist);
     if ((rc = ix->d_key.ensure(kbytes))) return rc;
     const bool want_id = out_id != nullptr;
-    if (want_id && ix->has_pos2id && !ix->d_pos2id.p) {  // first host-buffer call: the id table moves to the device
-        if ((rc = ix->d_pos2id.ensure(std::max<size_t>(ix->pos2id_host.size(), 1) * 4))) return rc;
-        CU(cudaMemcpyAsync(ix->d_pos2id.p, ix->pos2id_host.data(), ix->pos2id_host.size() * 4, cudaMemcpyHostToDevice, ix->stream));
-    }
+    if (want_id && (rc = upload_pos2id(ix))) return rc;
     rc = dpq_index_search_device(ix, reinterpret_cast<const float*>(dq), Q, topk, ix->d_key.as<uint64_t>());
     if (rc) return rc;
     dpq::launch_unpack(ix->d_key.as<uint64_t>(), nk, want_id && ix->has_pos2id ? ix->d_pos2id.as<uint32_t>() : nullptr,
@@ -1593,6 +1751,11 @@ int64_t dpq_index_stat(dpq_index* ix, const char* name) {
     if (n == "last_delete_us") return ix->last_delete_us;
     if (n == "n_added") return ix->n_added;
     if (n == "last_add_us") return ix->last_add_us;
+    if (n == "last_compact_us") return ix->compact_us[0];
+    if (n == "last_compact_gather_us") return ix->compact_us[1];
+    if (n == "last_compact_edge_us") return ix->compact_us[2];
+    if (n == "last_compact_layout_us") return ix->compact_us[3];
+    if (n == "last_compact_build_us") return ix->compact_us[2] + ix->compact_us[3];
     if (n.rfind("depth_hist_", 0) == 0) {
         size_t d = (size_t)atoi(n.c_str() + 11);
         return d < P.depth_hist.size() ? P.depth_hist[d] : 0;
@@ -1659,3 +1822,21 @@ int dpq_adc_tables(const float* cw, int M, int K, int Ds, const float* queries, 
 }
 
 }  // extern "C"
+
+namespace dpq {  // for dpq_multi_compact (multi.cu)
+int index_live_nodes(dpq_index* ix, uint8_t** d_codes, uint32_t** d_ids, int64_t* n_live) {
+    if (!ix->prog.v2)
+        return fail(DPQ_ERR_ARG, "dpq_multi_compact: compaction needs the code-array engine (this handle runs the first-generation engine, DPQ_ENGINE=1)");
+    CU(cudaSetDevice(ix->device));
+    return live_nodes(ix, d_codes, d_ids, n_live);
+}
+// A forest part compacted inside a multi-GPU handle: its id table (the global positions the handle gave its nodes)
+// moves to *ids, and the part reports positions as ids again, as every part of a handle does.
+void index_take_ids(dpq_index* ix, std::vector<uint32_t>* ids) {
+    ids->swap(ix->pos2id_host);
+    std::vector<uint32_t>().swap(ix->pos2id_host);
+    ix->has_pos2id = false;
+    cudaSetDevice(ix->device);
+    ix->d_pos2id.release();
+}
+}  // namespace dpq

@@ -13,12 +13,38 @@ static std::string base_name(const std::string& dataset, int M, int K) {
     return dataset + "/M" + std::to_string(M) + "K" + std::to_string(K);
 }
 
+static std::string nodes_file(const std::string& dataset, int M, int K, const std::string& sfx) {
+    return base_name(dataset, M, K) + "_Approx_TreeNodesDFS" + sfx + (M == 8 ? "" : ".vec_id");
+}
+static std::string tree_file(const std::string& dataset, int M, int K, const std::string& sfx) {
+    return base_name(dataset, M, K) + "_Approx_compressed_codes_opt" + sfx;
+}
+
+// the node file (QNode records at M = 8, else the position -> vec_id extension file) and the tree file with its
+// 16-byte header of a tree of N nodes, under the names of suffix `sfx`
+static int write_tree(const std::string& dataset, int M, int K, dpq_tree* t, long long N, const std::string& sfx) {
+    const std::string f_nodes = nodes_file(dataset, M, K, sfx), f_tree = tree_file(dataset, M, K, sfx);
+    if (M == 8) {  // QNode records exist for M == 8 only (DCAT.h:79-101)
+        std::vector<uint8_t> qn((size_t)dpq_tree_size(t, "qnodes"));
+        DPQ_TRY(dpq_tree_copy(t, "qnodes", qn.data()));
+        if (!write_file(f_nodes, nullptr, 0, qn.data(), qn.size())) return die("cannot write " + f_nodes);
+    } else {
+        std::vector<uint32_t> v((size_t)N);
+        DPQ_TRY(dpq_tree_copy(t, "vec_id", v.data()));
+        if (!write_file(f_nodes, nullptr, 0, v.data(), v.size() * 4)) return die("cannot write vec_id file");
+    }
+    std::vector<uint8_t> payload((size_t)dpq_tree_size(t, "payload"));
+    DPQ_TRY(dpq_tree_copy(t, "payload", payload.data()));
+    int64_t hdr[2] = {(int64_t)N, (int64_t)payload.size()};  // DCAT.h:1840-1842
+    if (!write_file(f_tree, hdr, 16, payload.data(), payload.size())) return die("cannot write " + f_tree);
+    std::cout << "n_diffs " << dpq_tree_size(t, "n_diffs") << " number of bytes " << payload.size() << std::endl;
+    return 0;
+}
+
 // one tree: `codes` [n][M] -> the three files of create_approx_tree (DCAT.h:970-1065) with suffix `sfx`
 static int build_one(const std::string& dataset, int M, int K, int H, int method, const uint8_t* codes, long long N,
                      const Codebook& cb, const std::string& sfx) {
     const std::string f_edges = base_name(dataset, M, K) + "H" + std::to_string(H) + "_Approx_Edges" + sfx;
-    const std::string f_nodes = base_name(dataset, M, K) + "_Approx_TreeNodesDFS" + sfx;
-    const std::string f_tree = base_name(dataset, M, K) + "_Approx_compressed_codes_opt" + sfx;
     dpq_tree* t = nullptr;
     if (file_exists(f_edges)) {  // stage caching by file existence (DCAT.h:1230-1242)
         std::vector<uint32_t> e((size_t)(2 * (N - 1) + 1));
@@ -35,22 +61,9 @@ static int build_one(const std::string& dataset, int M, int K, int H, int method
         if (N > 1) DPQ_TRY(dpq_tree_copy(t, "edges", e.data() + 1));
         if (!write_file(f_edges, nullptr, 0, e.data(), e.size() * 4)) return die("cannot write " + f_edges);
     }
-    if (M == 8) {  // QNode records exist for M == 8 only (DCAT.h:79-101)
-        std::vector<uint8_t> qn((size_t)dpq_tree_size(t, "qnodes"));
-        DPQ_TRY(dpq_tree_copy(t, "qnodes", qn.data()));
-        if (!write_file(f_nodes, nullptr, 0, qn.data(), qn.size())) return die("cannot write " + f_nodes);
-    } else {  // extension: position -> vec_id only
-        std::vector<uint32_t> v((size_t)N);
-        DPQ_TRY(dpq_tree_copy(t, "vec_id", v.data()));
-        if (!write_file(f_nodes + ".vec_id", nullptr, 0, v.data(), v.size() * 4)) return die("cannot write vec_id file");
-    }
-    std::vector<uint8_t> payload((size_t)dpq_tree_size(t, "payload"));
-    DPQ_TRY(dpq_tree_copy(t, "payload", payload.data()));
-    int64_t hdr[2] = {(int64_t)N, (int64_t)payload.size()};  // DCAT.h:1840-1842
-    if (!write_file(f_tree, hdr, 16, payload.data(), payload.size())) return die("cannot write " + f_tree);
-    std::cout << "n_diffs " << dpq_tree_size(t, "n_diffs") << " number of bytes " << payload.size() << std::endl;
+    const int rc = write_tree(dataset, M, K, t, N, sfx);
     dpq_tree_free(t);
-    return 0;
+    return rc;
 }
 
 // -parts P (extension, the 1B-code layout): part p = vector ids [p*N/P, (p+1)*N/P), its own tree,
@@ -124,7 +137,7 @@ static int query(const Args& a, const std::string& dataset, const std::string& e
     std::vector<float> q((size_t)nq * Dp, 0.f);
     for (long long i = 0; i < nq; ++i) memcpy(&q[i * Dp], &raw[i * D], (size_t)D * 4);
     const std::string sfx = method_suffix(method) + "_N" + std::to_string(N);
-    const std::string f_tree = base_name(dataset, M, K) + "_Approx_compressed_codes_opt" + sfx;
+    const std::string f_tree = tree_file(dataset, M, K, sfx);
     const std::string f_nodes = base_name(dataset, M, K) + "_Approx_TreeNodesDFS" + sfx;
     // -gpus N (extension): the tree is sharded by depth-1 subtrees over N GPUs of this box, the
     // per-GPU top-k lists are all-gathered over NCCL and merged (dpq_multi_*, SURVEY 8e)
@@ -133,6 +146,8 @@ static int query(const Args& a, const std::string& dataset, const std::string& e
     const char* nodes_arg = (M == 8 && file_exists(f_nodes)) ? f_nodes.c_str() : nullptr;
     std::vector<uint32_t> pos((size_t)nq * top_k), id(pos.size());
     std::vector<float> dist(pos.size());
+    const bool compact = a.has("-compact");
+    if (compact && (P > 1 || n_gpus > 1)) return die("-compact works on the single-GPU index only (not with -gpus or -parts)");
     dpq_index* ix = nullptr;
     dpq_multi* mx = nullptr;
     if (P > 1) {
@@ -183,6 +198,21 @@ static int query(const Args& a, const std::string& dataset, const std::string& e
         if (mx) DPQ_TRY(dpq_multi_delete(mx, del.data(), (int64_t)del.size()));
         else DPQ_TRY(dpq_index_delete(ix, del.data(), (int64_t)del.size()));
     }
+    if (compact) {  // extension: the tree rebuilt over the live nodes, written as the files of -method 1 -N <live count>
+        dpq_tree* t = nullptr;
+        DPQ_TRY(dpq_index_compact(ix, &t));
+        const long long n_live = dpq_tree_size(t, "n_codes");
+        const std::string csfx = method_suffix(1) + "_N" + std::to_string(n_live);  // the compaction builds with -method 1
+        for (const std::string& f : {nodes_file(dataset, M, K, csfx), tree_file(dataset, M, K, csfx)})
+            if (file_exists(f)) {
+                dpq_tree_free(t);
+                return die("-compact: " + f + " exists and is not overwritten");
+            }
+        const int rc = write_tree(dataset, M, K, t, n_live, csfx);
+        dpq_tree_free(t);
+        if (rc) return rc;
+        std::cout << "compacted: " << n_live << " live nodes, query them with -method 1 -N " << n_live << std::endl;
+    }
     const int reps = (int)a.num("-repeat", 1);  // extension: repeat the batch (the first call pays allocations)
     double t0 = now_s();
     for (int it = 0; it < reps; ++it) {
@@ -214,7 +244,7 @@ int main(int argc, char** argv) {
     Args a{argc, argv};
     std::string dataset = a.str("-dataset", ""), ext = a.str("-ext", "fvecs"), task = a.str("-task", "approx_tree");
     int M = (int)a.num("-m", 8), K = (int)a.num("-k", 256);
-    if (dataset.empty()) return die("usage: deltapq -dataset DIR -task approx_tree|query|query_im|batch_query -m M -k K -h 1 -diff M -N N [-query_size Q] [-topk k] [-method 1|2] [-debug] [-results FILE] [-gpus N] [-parts P] [-repeat R] [-add FILE] [-deleted FILE]");
+    if (dataset.empty()) return die("usage: deltapq -dataset DIR -task approx_tree|query|query_im|batch_query -m M -k K -h 1 -diff M -N N [-query_size Q] [-topk k] [-method 1|2] [-debug] [-results FILE] [-gpus N] [-parts P] [-repeat R] [-add FILE] [-deleted FILE] [-compact (writes the files of -method 1 -N <live count>)]");
     if (task == "approx_tree") return approx_tree(a, dataset, M, K);
     if (task == "query" || task == "query_im" || task == "batch_query") return query(a, dataset, ext, M, K);
     return die("deltapq: task '" + task + "' is outside the B200 hot-path scope (approx_tree, query, query_im, batch_query)");

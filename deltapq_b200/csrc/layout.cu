@@ -377,7 +377,7 @@ int depth_hist_device(int device, const uint8_t* d_depth, int64_t n, int64_t* hi
 }
 
 int layout_tree_device(const uint8_t* codes, int64_t n, int M, int K, const float* cw, int Ds, dpq_tree* t,
-                       const uint32_t* d_edges_in, bool keep_on_device) {
+                       const uint32_t* d_edges_in, bool keep_on_device, bool keep_qnode_fields) {
     int rc = api_check_device();
     if (rc) return rc;
     CU(cudaSetDevice(api_device()));
@@ -527,6 +527,16 @@ int layout_tree_device(const uint8_t* codes, int64_t n, int M, int K, const floa
         int64_t hist[17];
         if ((rc = depth_hist_device(api_device(), d_depthp.as<uint8_t>(), n, hist))) return rc;
         t->depth_hist.assign(hist, hist + 17);
+        if (keep_qnode_fields) {  // what the QNode records need beyond the device arrays
+            t->parent_pos.resize((size_t)n);
+            t->child_num.resize((size_t)n);
+            t->max_dist.resize((size_t)n);
+            t->max_dist2p.resize((size_t)n);
+            CU(cudaMemcpy(t->parent_pos.data(), d_ppos.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(t->child_num.data(), d_cnum.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(t->max_dist.data(), d_md.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(t->max_dist2p.data(), d_md2.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
+        }
         CU(cudaDeviceSynchronize());
         t->on_device = true;
         t->device = api_device();

@@ -23,6 +23,8 @@
 namespace dpq {
 int api_fail(int code, const std::string& msg);
 int api_check_device();
+int index_live_nodes(dpq_index* ix, uint8_t** d_codes, uint32_t** d_ids, int64_t* n_live);  // api.cu
+void index_take_ids(dpq_index* ix, std::vector<uint32_t>* ids);
 }
 
 namespace {
@@ -80,6 +82,8 @@ struct dpq_multi {
     size_t h_cap = 0;
     std::vector<uint32_t> pos2id;  // position -> vector id over the whole position space
     size_t last = 0;               // the index whose positions end the position space: it takes every add
+    bool forest = false;           // dpq_multi_open_parts: ix are forest parts, else subtree shards of one tree
+    std::vector<float> cw;         // the codebook: dpq_multi_compact builds a tree with it
     int64_t open_us = 0, nccl_us = 0;  // wall time of opening the shards / of ncclCommInitAll
 };
 
@@ -233,6 +237,7 @@ int dpq_multi_open_parts(const char* const* tree_paths, const char* const* qnode
     dpq_multi* m = nullptr;
     int rc = begin_multi_open(n_gpus, n_parts, M, K, &m);
     if (rc) return rc;
+    m->forest = true;
     int64_t span = 0;
     {
         // parts are dealt round-robin to the GPUs and opened concurrently: the host decode of a stream is
@@ -287,6 +292,7 @@ int dpq_multi_open_parts(const char* const* tree_paths, const char* const* qnode
 int dpq_multi_set_codebook(dpq_multi* m, const float* codewords, int Ds) {
     if (!m || !codewords) return dpq::api_fail(DPQ_ERR_ARG, "dpq_multi_set_codebook: null");
     m->Ds = Ds;
+    m->cw.assign(codewords, codewords + (size_t)m->M * m->K * Ds);
     for (size_t i = 0; i < m->ix.size(); ++i) {
         CUM(cudaSetDevice(m->dev[i]));
         int rc = dpq_index_set_codebook(m->ix[i], codewords, Ds);
@@ -463,6 +469,122 @@ int dpq_multi_add(dpq_multi* m, const uint8_t* codes, int64_t n, const uint32_t*
 }
 int dpq_multi_add_vectors(dpq_multi* m, const float* x, int64_t n, int D, const uint32_t* ids, uint32_t* out_pos) {
     return multi_add(m, x, n, D < 1 ? -1 : D, ids, out_pos, "dpq_multi_add_vectors");
+}
+
+// The handle reports ids through its table, indexed by global position; a position it does not cover is its own id.
+static uint32_t id_of(const std::vector<uint32_t>& tab, uint32_t pos) { return pos < tab.size() ? tab[pos] : pos; }
+
+// Forest parts: each part is compacted in place on its GPU (dpq_index_compact keeps first_pos); the ids it carries
+// are the global positions the handle knew, translated through the old table into the new one part by part, so a
+// failure in a later part leaves a consistent handle.
+static int compact_parts(dpq_multi* m) {
+    int64_t span = 0;
+    for (size_t p = 0; p < m->ix.size(); ++p) {
+        const int64_t live = dpq_index_stat(m->ix[p], "n_local") - dpq_index_stat(m->ix[p], "n_deleted");
+        if (live < 1) return dpq::api_fail(DPQ_ERR_ARG, "dpq_multi_compact: part " + std::to_string(p) + " has no live node");
+        span = std::max(span, dpq_index_stat(m->ix[p], "base_pos") + dpq_index_stat(m->ix[p], "n_local"));
+    }
+    const std::vector<uint32_t> old = m->pos2id;
+    if (m->pos2id.size() < (size_t)span) {
+        const size_t from = m->pos2id.size();
+        m->pos2id.resize((size_t)span);
+        for (size_t i = from; i < m->pos2id.size(); ++i) m->pos2id[i] = (uint32_t)i;
+    }
+    for (size_t p = 0; p < m->ix.size(); ++p) {
+        dpq_index* ix = m->ix[p];
+        const int64_t first = dpq_index_stat(ix, "base_pos"), n_old = dpq_index_stat(ix, "n_local");
+        CUM(cudaSetDevice(m->dev[p]));
+        int rc = dpq_index_compact(ix, nullptr);
+        if (rc) return rc;
+        std::vector<uint32_t> ids;
+        dpq::index_take_ids(ix, &ids);
+        for (size_t i = 0; i < ids.size(); ++i) m->pos2id[(size_t)first + i] = id_of(old, ids[i]);
+        for (int64_t q = first + (int64_t)ids.size(); q < first + n_old; ++q) m->pos2id[(size_t)q] = (uint32_t)q;  // no node
+    }
+    CUM(cudaSetDevice(0));
+    return DPQ_OK;
+}
+
+// Subtree shards: every shard's live codes and positions are gathered on its GPU, copied in rank order (= global
+// position order) to GPU 0, built into one tree there, and its stream is dealt to the GPUs again as
+// dpq_multi_open_file deals a file.  The new shards replace the old ones only once all of them are open.
+static int compact_shards(dpq_multi* m) {
+    const size_t n = m->ix.size();
+    std::vector<uint8_t*> codes(n, nullptr);
+    std::vector<uint32_t*> pos(n, nullptr);
+    std::vector<int64_t> cnt(n, 0);
+    std::vector<dpq_index*> fresh(n, nullptr);
+    uint8_t* all_codes = nullptr;
+    uint32_t* all_pos = nullptr;
+    dpq_tree* t = nullptr;
+    auto cleanup = [&](int rc) {
+        for (size_t r = 0; r < n; ++r) {
+            cudaSetDevice(m->dev[r]);
+            if (codes[r]) cudaFree(codes[r]);
+            if (pos[r]) cudaFree(pos[r]);
+            if (fresh[r]) dpq_index_close(fresh[r]);
+        }
+        cudaSetDevice(0);
+        if (all_codes) cudaFree(all_codes);
+        if (all_pos) cudaFree(all_pos);
+        dpq_tree_free(t);
+        (void)cudaGetLastError();
+        dpq_set_device(0);
+        return rc;
+    };
+    const std::string keep_err = "dpq_multi_compact: ";
+    auto cuda_fail = [&](cudaError_t e) { return cleanup(dpq::api_fail(DPQ_ERR_CUDA, keep_err + cudaGetErrorString(e))); };
+    int64_t total = 0;
+    for (size_t r = 0; r < n; ++r) {
+        int rc = dpq::index_live_nodes(m->ix[r], &codes[r], &pos[r], &cnt[r]);  // shards have no id table: ids = positions
+        if (rc) return cleanup(rc);
+        total += cnt[r];
+    }
+    if (total == 0) return cleanup(dpq::api_fail(DPQ_ERR_ARG, "dpq_multi_compact: every node is deleted (a tree needs at least one node)"));
+    const int M = m->M, K = m->K;
+    int rc = dpq_set_device(0);
+    if (rc) return cleanup(rc);
+    cudaError_t e = cudaMalloc(&all_codes, (size_t)total * M);
+    if (e == cudaSuccess) e = cudaMalloc(&all_pos, (size_t)total * 4);
+    for (size_t r = 0, off = 0; r < n && e == cudaSuccess; off += (size_t)cnt[r], ++r) {
+        if (!cnt[r]) continue;  // another GPU's memory: peer or host-staged copies, whatever the platform has
+        e = cudaMemcpyAsync(all_codes + off * M, codes[r], (size_t)cnt[r] * M, cudaMemcpyDefault, m->st[0]);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(all_pos + off, pos[r], (size_t)cnt[r] * 4, cudaMemcpyDefault, m->st[0]);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(m->st[0]);
+    if (e != cudaSuccess) return cuda_fail(e);
+    if ((rc = dpq_tree_build_device(all_codes, total, M, K, m->cw.data(), m->Ds, 1, 1, &t))) return cleanup(rc);
+    std::vector<uint8_t> payload((size_t)dpq_tree_size(t, "payload"));
+    std::vector<uint32_t> row((size_t)total), old_pos((size_t)total);
+    if ((rc = dpq_tree_copy(t, "payload", payload.data())) || (rc = dpq_tree_copy(t, "vec_id", row.data()))) return cleanup(rc);
+    if ((e = cudaMemcpy(old_pos.data(), all_pos, (size_t)total * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) return cuda_fail(e);
+    std::vector<uint32_t> tab((size_t)total);
+    for (size_t p = 0; p < tab.size(); ++p) tab[p] = id_of(m->pos2id, old_pos[row[p]]);
+    for (size_t r = 0; r < n; ++r) {
+        if ((rc = dpq_set_device(m->dev[r])) ||
+            (rc = dpq_index_open(payload.data(), (int64_t)payload.size(), total, M, K, nullptr, (int)r, (int)n, &fresh[r])) ||
+            (rc = dpq_index_set_codebook(fresh[r], m->cw.data(), m->Ds)) || (rc = dpq_index_set_stream(fresh[r], m->st[r])))
+            return cleanup(rc);
+    }
+    for (size_t r = 0; r < n; ++r) {
+        cudaSetDevice(m->dev[r]);
+        dpq_index_close(m->ix[r]);
+        m->ix[r] = fresh[r];
+        fresh[r] = nullptr;
+    }
+    m->pos2id.swap(tab);
+    return cleanup(DPQ_OK);
+}
+
+int dpq_multi_compact(dpq_multi* m) {
+    int rc = dpq::api_check_device();
+    if (rc) return rc;
+    if (!m) return dpq::api_fail(DPQ_ERR_ARG, "dpq_multi_compact: null handle");
+    if (m->Ds < 1 || m->cw.empty()) return dpq::api_fail(DPQ_ERR_ARG, "dpq_multi_compact: codebook not set");
+    for (dpq_index* ix : m->ix)  // checked for every index first: the handle stays unchanged
+        if (dpq_index_stat(ix, "engine") != 2)
+            return dpq::api_fail(DPQ_ERR_ARG, "dpq_multi_compact: compaction needs the code-array engine (this handle runs the first-generation engine, DPQ_ENGINE=1)");
+    return m->forest ? compact_parts(m) : compact_shards(m);
 }
 
 int64_t dpq_multi_stat(dpq_multi* m, int rank, const char* name) {

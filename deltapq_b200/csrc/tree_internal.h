@@ -37,9 +37,10 @@ void centroid_tables(const float* cw, int M, int K, int Ds, std::vector<float>& 
 // DFS layout + stream on the GPU (layout.cu): fills every array of *t from t->edges / t->root.
 // codes: [n][M] host pointer.  Returns 0 or a DPQ_ERR_* code (text via dpq_last_error).
 // d_edges: the edges already on the device (uint32 [n-1][2]) or nullptr to upload t->edges; keep_on_device:
-// leave the result in HBM (dpq_tree::on_device) instead of copying every array to the host.
+// leave the result in HBM (dpq_tree::on_device) instead of copying every array to the host; keep_qnode_fields (with
+// keep_on_device): also copy parent_pos, child_num, max_dist and max_dist2p to the host vectors (dpq_index_compact).
 int layout_tree_device(const uint8_t* codes, int64_t n, int M, int K, const float* cw, int Ds, dpq_tree* t,
-                       const uint32_t* d_edges = nullptr, bool keep_on_device = false);
+                       const uint32_t* d_edges = nullptr, bool keep_on_device = false, bool keep_qnode_fields = false);
 // edge search with the result left on the device: *d_edges_out is a cudaMalloc'ed uint32 [n-1][2] array the
 // caller frees; codes may be a host or a device pointer (edges.cu)
 int find_edges_device(const uint8_t* codes, int64_t n, int M, int K, int max_height_folds, int method,

@@ -114,7 +114,8 @@ int dpq_index_set_option(dpq_index* idx, const char* name, int64_t value);
  * fewer than topk nodes are live.  The bitmap (one bit per node of the shard) appears on the first delete.
  * dpq_index_undelete clears the same bits; once nothing is deleted the index answers exactly as one that never
  * had deletions.  The call runs on the index's stream (the caller's after dpq_index_set_stream) and returns
- * once the change is complete: every search issued after it sees it.  Deletions are not written to any file.
+ * once the change is complete: every search issued after it sees it.  Deletions reach a file through
+ * dpq_index_compact, which drops the deleted nodes from a rebuilt tree.
  * The first-generation engine (DPQ_ENGINE=1) has no deletion: DPQ_ERR_ARG.  Stat "n_deleted": nodes of this
  * shard currently deleted; "last_delete_us": host wall time of the last call. */
 int dpq_index_delete(dpq_index* idx, const uint32_t* ids, int64_t n);
@@ -139,10 +140,31 @@ int dpq_index_undelete(dpq_index* idx, const uint32_t* ids, int64_t n);
  * Ids: an index without a pos2id table keeps none while ids is NULL (id = position); the first add that names
  * ids creates one, identity over the nodes it already had.  Duplicate ids are allowed: dpq_index_delete removes
  * every node that carries the id, and a node added after its id was deleted is live (the bitmap is per node).
- * The call runs on the index's stream and returns once the change is complete.  Adds are not written to any
- * file.  Stats: "n_added" (appended nodes), "last_add_us"; "n_local" counts appended nodes, "n_codes" does not. */
+ * The call runs on the index's stream and returns once the change is complete.  Adds reach a file through
+ * dpq_index_compact, which builds them into the tree.  Stats: "n_added" (appended nodes), "last_add_us"; "n_local" counts appended nodes, "n_codes" does not. */
 int dpq_index_add(dpq_index* idx, const uint8_t* codes, int64_t n, const uint32_t* ids, uint32_t* out_pos);
 int dpq_index_add_vectors(dpq_index* idx, const float* x, int64_t n, int D, const uint32_t* ids, uint32_t* out_pos);
+
+/* Compacts an open index (an extension, like deletion and adds; the reference rebuilds its trees): the live nodes,
+ * tree nodes and appended ones alike, are gathered on the device in ascending position, a new DeltaTree is built
+ * over them on the device (the edge search and layout of dpq_tree_build_device with -h 1, -method 1 and this
+ * index's codebook), and it replaces the index's tree.  Afterwards no node is deleted or appended: n_codes = n_local
+ * = the live count, and n_bytes, n_diffs, n_chunks and the depth histogram are the new tree's.
+ * Positions are renumbered: the new tree's DFS order, from the same base_pos (a forest part keeps first_pos).
+ * Ids are not: every node reports the id it reported before, and the index always has an id table afterwards (an
+ * index that had none reports each node's old position as its id).  Deletions, adds and searches continue on the
+ * new tree as on any other (adds take the positions after the live count).  Options, stream and codebook are kept.
+ * out_tree (may be NULL) receives the new tree as dpq_tree_build(live codes) returns it, vec_id mapped to the ids:
+ * "payload", "vec_id", "depth", "codes_by_pos", "n_codes", "n_diffs" and, at M = 8, "qnodes" (vec_id field = the
+ * id), which are the bytes of the reference's files; the caller writes them and frees the tree with dpq_tree_free.
+ * Without out_tree nothing but the index's own id table leaves the device.
+ * DPQ_ERR_ARG, index unchanged: a shard of a tree split over n_ranks > 1 (dpq_multi_compact), no codebook, the
+ * first-generation engine (DPQ_ENGINE=1), no live node.  Any failure (e.g. out of memory during the edge search)
+ * leaves the index unchanged and searchable.  The gather runs on the index's stream, the build on the device's
+ * legacy stream; the call returns once everything is complete.  Stats: "last_compact_us" (host wall time),
+ * "last_compact_gather_us", "last_compact_edge_us", "last_compact_layout_us", "last_compact_build_us" (edge search
+ * + layout). */
+int dpq_index_compact(dpq_index* idx, struct dpq_tree** out_tree);
 
 /* Replaces the per-query loop dmain:328-344 calling
  * query_processing_scan_compressed_codes_opt_o_direct (DCAT.h:2805) /
@@ -196,9 +218,18 @@ int dpq_multi_undelete(dpq_multi* m, const uint32_t* ids, int64_t n);
  * (the last shard, or the part with the largest first_pos) and the new positions continue the global space.
  * The handle's id table grows with them (created as identity when it was empty and ids are given), so that
  * dpq_multi_search reports the ids and dpq_multi_delete takes them.  As for dpq_index_add, the inputs may be on
- * any device.  Every add lands on that one GPU: a known imbalance of the search load. */
+ * any device.  Every add lands on that one GPU, a known imbalance of the search load until dpq_multi_compact. */
 int dpq_multi_add(dpq_multi* m, const uint8_t* codes, int64_t n, const uint32_t* ids, uint32_t* out_pos);
 int dpq_multi_add_vectors(dpq_multi* m, const float* x, int64_t n, int D, const uint32_t* ids, uint32_t* out_pos);
+/* dpq_index_compact for the handle (dpq_multi_set_codebook first).  Subtree shards (dpq_multi_open_file): the live
+ * nodes of every shard are gathered in global position order onto GPU 0, one tree is built there and dealt to the
+ * GPUs again by whole depth-1 subtrees balanced by stream bytes, as dpq_multi_open_file deals a file, so appended
+ * nodes are spread over every GPU.  Forest parts (dpq_multi_open_parts): every part is compacted in place on its
+ * GPU and keeps its first_pos.  Positions are renumbered, ids kept (the handle's id table is rebuilt; without one
+ * before, a node's id is its old global position).  DPQ_ERR_ARG, handle unchanged: no codebook, the first-generation
+ * engine (DPQ_ENGINE=1), no live node (shards) or a part without a live node (parts).  With n_gpus > 1 the gather
+ * onto GPU 0 copies across devices with cudaMemcpyAsync (peer or host-staged). */
+int dpq_multi_compact(dpq_multi* m);
 void dpq_multi_close(dpq_multi* m);
 
 /* Raw device allocation helpers for hosts without a CUDA binding (ctypes, cgo, JNI). */
@@ -218,7 +249,8 @@ int dpq_free_host(void* hptr);
  * "last_coarse" (1 when the last search used the sample -> 8-bit coarse scan -> exact re-score
  * path), "last_latency" (1: latency mode), "last_scan8_us" / "sum_scan8_ns" (the coarse scan kernel
  * alone; in latency mode the full scan1 pass), "device_bytes_per_node", "engine"; "n_deleted",
- * "last_delete_us" (dpq_index_delete); "n_added", "last_add_us" (dpq_index_add). */
+ * "last_delete_us" (dpq_index_delete); "n_added", "last_add_us" (dpq_index_add); "last_compact_us" and its stages
+ * (dpq_index_compact). */
 int64_t dpq_index_stat(dpq_index* idx, const char* name);
 
 void dpq_index_close(dpq_index* idx);
