@@ -67,15 +67,18 @@ __global__ void __launch_bounds__(256) lut_kernel(const float* __restrict__ cw, 
     double sum = 0.0;
     for (int m = 0; m < M; ++m) sum += (double)__int_as_float(s_max[m]);
     const double qmax = g.pack == 1 ? (double)(1u << 30) : (double)(32767 - 16);
-    const double s = sum > 0.0 ? qmax / sum : 1.0;
+    // a sum that is not positive (NaN from a NaN query component, or 0) scales by 0, as an infinite one does: every
+    // entry 0, a filter that passes every node, the exact re-score and fallback decide
+    const double s = sum > 0.0 ? qmax / sum : 0.0;
     if (k == 0) {
         scale[vq] = s;
         gthr[vq] = g.pack == 1 ? kInf31 : 0x8000u;
     }
-    // rows beyond M*K are never addressed; entry (m,k) lives at word (row ^ lane)
+    // rows beyond M*K are never addressed; entry (m,k) lives at word (row ^ lane).  Every entry is clamped to
+    // [0, qmax] before packing (a no-op for a finite positive sum; NaN -> 0): no value can leave its lane.
     if (k < K)
         for (int m = 0; m < M; ++m) {
-            uint32_t v = (uint32_t)__double2ll_rn((double)out[m * K + k] * s);
+            uint32_t v = (uint32_t)__double2ll_rn(fmin(fmax((double)out[m * K + k] * s, 0.0), qmax));
             int r = (m * K + k) ^ lane;
             if (g.pack == 1) dst[r] = v;
             else reinterpret_cast<uint16_t*>(dst)[2 * r + half] = (uint16_t)v;

@@ -58,11 +58,16 @@ __global__ void __launch_bounds__(S1_T, 1) scan1_kernel(const Scan1Args a) {
     const bool live1 = q1 < a.Q;
     const int MK = a.M * a.K;
     // fixed-point scale of each query: 65500 / sum of the per-subspace maxima, so that a node's M entries
-    // sum below 2^16 (+ M/2 of rounding)
+    // sum below 2^16 (+ M/2 of rounding).  A sum that is not finite and positive (a NaN or infinite query
+    // component) scales by 0: every entry 0, the filter passes every node and the exact re-score decides.
     auto scale_of = [&](int q) -> double {
         double sum = 0.0;
         for (int m = 0; m < a.M; ++m) sum += (double)a.mmax[q * 16 + m];
-        return sum > 0.0 ? 65500.0 / sum : 1.0;
+        return sum > 0.0 ? 65500.0 / sum : 0.0;
+    };
+    // entries clamped to the lane's range before packing (NaN -> 0): no value reaches the partner's half
+    auto entry = [&](int q, int i, double sc) -> uint32_t {
+        return (uint32_t)__double2int_rn(fmin(fmax((double)a.lutf[(size_t)q * MK + i] * sc, 0.0), 65500.0));
     };
     const double sc0 = scale_of(q0);
     const double sc1 = live1 ? scale_of(q1) : 0.0;
@@ -70,8 +75,8 @@ __global__ void __launch_bounds__(S1_T, 1) scan1_kernel(const Scan1Args a) {
         const int m = e >> 8, c = e & 255;
         uint32_t w = 0;
         if (m < a.M && c < a.K) {
-            const uint32_t v0 = (uint32_t)__double2int_rn((double)a.lutf[(size_t)q0 * MK + m * a.K + c] * sc0);
-            const uint32_t v1 = live1 ? (uint32_t)__double2int_rn((double)a.lutf[(size_t)q1 * MK + m * a.K + c] * sc1) : 0u;
+            const uint32_t v0 = entry(q0, m * a.K + c, sc0);
+            const uint32_t v1 = live1 ? entry(q1, m * a.K + c, sc1) : 0u;
             w = v0 | (v1 << 16);
         }
         uint4* dst = reinterpret_cast<uint4*>(table + (size_t)e * 64);

@@ -144,7 +144,7 @@ __global__ void scale2_kernel(const float* __restrict__ mmax, int M, int Q, doub
     if (q >= Q) return;
     double sum = 0.0;
     for (int m = 0; m < M; ++m) sum += (double)mmax[(size_t)q * 16 + m];
-    scale[q] = sum > 0.0 ? (double)(32767 - 16) / sum : 1.0;
+    scale[q] = sum > 0.0 ? (double)(32767 - 16) / sum : 0.0;  // NaN or 0: scale 0, the filter passes every node
 }
 
 // Small batches (latency mode): one block per (query, subspace), so that even a single query spreads
@@ -191,7 +191,10 @@ __global__ void __launch_bounds__(256) pack2_kernel(const float* __restrict__ lu
         const int q = grp * QB + ql, row = row0 + r;
         uint16_t v = 0;
         const int m = row >> 8, c = row & 255;  // scan-table row = m * 256 + centroid
-        if (q < Q && m < M && c < K) v = (uint16_t)__double2ll_rn((double)lutf[(size_t)q * MK + m * K + c] * scale[q]);
+        // clamped to the 15-bit range scale2_kernel scales to (a no-op for a finite positive sum; NaN -> 0): no
+        // entry can wrap into bit 15 and carry or borrow into the neighbouring query's lane
+        if (q < Q && m < M && c < K)
+            v = (uint16_t)__double2ll_rn(fmin(fmax((double)lutf[(size_t)q * MK + m * K + c] * scale[q], 0.0), 32767.0 - 16.0));
         tile[r * QB + ql] = v;
     }
     __syncthreads();
